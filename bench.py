@@ -30,6 +30,10 @@ parity_vs_golden
          (tests/golden/gcg_reference.json: p1_fem_kuhn m = 12 nev = 10 and m = 24 nev = 200) and the line
          carries iteration counts, eigenvalue differences and whether all ranks hold identical bits.
 
+--dump-outputs DIR
+         after the timed steps, what the last timed solve handed its caller goes to DIR as .npy files (see
+         dump_outputs); inputs are generated from fixed seeds, so two builds can be compared output for output.
+
 Other workloads of BASELINE.json (same line format): --workload laplace7 --m 100 --nev 50 (config 2,
 standard problem, analytic eigenvalues as the parity pin), --workload q1_27pt (config 4's operator), and
 --kernel-sweep (config 5: per-kernel sweep at n = m^3, k = 16 ... 512, with the reference's slots timed on the host
@@ -57,8 +61,8 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 
-# outer iterations the full workload needs (measured on B200 with this repo, recorded by
-# bench.py itself into profiles/bench_iters.json); the reference arm scales its bounded
+# outer iterations the full workload needs (measured on B200 with this repo, kept in
+# profiles/bench_iters.json; bench.py only reads it); the reference arm scales its bounded
 # sample with it.  Iteration-count parity with the reference is a tested property (tests/).
 ITERS_FILE = ROOT / "profiles" / "bench_iters.json"
 
@@ -376,9 +380,36 @@ def golden_parity(api, dist, cases=(4, 9)) -> list:
     return out
 
 
+DUMP_EVEC_BYTES = 48 << 20          # eigenvector sample; with the eigenvalues the dump stays under 64 MB
+
+
+def dump_outputs(out_dir: Path, out: dict, evec, nev: int) -> None:
+    """--dump-outputs: the last timed solve's results as its caller receives them -- eigenvalues.npy (the nev
+    wanted eigenvalues), eigenvectors_sample.npy (their eigenvectors on a fixed set of rows: every row when that fits
+    DUMP_EVEC_BYTES, else rows drawn by numpy.random.default_rng(0) without replacement, ascending), num_iter.npy and
+    nev_conv.npy (scalars); all float64."""
+    n = evec.nrows
+    if n * 8 * nev <= DUMP_EVEC_BYTES:
+        rows = np.arange(n)
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_EVEC_BYTES // (8 * nev), replace=False))
+    sample = np.empty((rows.size, nev))
+    chunk = max(1, (256 << 20) // (8 * n))             # columns per download: ~256 MB of host memory, one column if larger
+    for c0 in range(0, nev, chunk):
+        c1 = min(nev, c0 + chunk)
+        sample[:, c0:c1] = evec.numpy(c0, c1)[rows]
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "eigenvalues.npy", np.asarray(out["eval"][:nev], dtype=np.float64))
+    np.save(out_dir / "eigenvectors_sample.npy", sample)
+    np.save(out_dir / "num_iter.npy", np.float64(out["num_iter"]))
+    np.save(out_dir / "nev_conv.npy", np.float64(out["nev_conv"]))
+
+
 # ------------------------------------------------------------------------------------- ours
 def run_b200(a) -> int:
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
+    if a.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes a single GPU's results: run bench.py as one process, without torchrun")
     import torch
     dist = None
     if world > 1:
@@ -469,6 +500,8 @@ def run_b200(a) -> int:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         sec = float(t.item())
     stats = out["stats"]
+    if a.dump_outputs:                                        # before the e2e solves below overwrite evec
+        dump_outputs(Path(a.dump_outputs), out, evec, a.nev)
 
     # ---- parity at full size, outside the timed region: every returned pair against the reference's
     # own acceptance test (src/ops_eig_sol_gcg.c:229-252): ||A x - lambda B x||_2 <= tol[0] and
@@ -583,14 +616,6 @@ def run_b200(a) -> int:
                 cores = host_cores()
                 m_s = min(a.same_m, a.m)
                 s = reference_sample(a.workload, a.nev, m_s, a.ref_iters, cores)
-                try:
-                    ITERS_FILE.parent.mkdir(exist_ok=True)
-                    d = json.loads(ITERS_FILE.read_text()) if ITERS_FILE.exists() else {}
-                    if a.max_iter <= 0 and a.workload == "p1_fem":
-                        d[f"m{a.m}_nev{a.nev}"] = {"num_iter": int(out["num_iter"]), "nev_conv": int(out["nev_conv"])}
-                        ITERS_FILE.write_text(json.dumps(d, indent=1, sort_keys=True) + "\n")
-                except Exception:
-                    pass
                 v, desc = scale_reference(s, a.m, a.nev)
                 cpu = {"value": v, "unit": "s", "cores": cores, "kind": "reference", "sample": desc}
                 # the device solver on the very same pencil, in the same run: a measured pair
@@ -686,7 +711,13 @@ def main() -> int:
     ap.add_argument("--sweep-cpu-m", type=int, default=64, help="lattice size of the CPU slices of --kernel-sweep")
     ap.add_argument("--ref-budget", type=float, default=240.0, help="--impl reference: seconds the one real solve may take")
     ap.add_argument("--ref-big-m", type=int, default=0, help="--impl reference: lattice size of the real solve (0: pick by budget)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed solve's eigenvalues, a "
+                    "fixed row sample of its eigenvectors and its iteration counts to DIR as .npy (single GPU)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.kernel_sweep):
+        ap.error("--dump-outputs applies to the timed device solve (--impl b200, no --kernel-sweep)")
     if a.workload == "cube4":
         a.m = 15
         a.same_m = 15

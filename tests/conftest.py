@@ -58,6 +58,27 @@ def reference_runs_over_threads(refmod, solve, threads=(1, 2, 4, 8)):
     return runs
 
 
+def recorded_reference_runs(generator, args, nev, nev_max, nev_init):
+    """The reference's own runs of one solve at 1, 2, 4 and 8 OpenMP threads as recorded in
+    tests/golden/reference_iteration_spread.json: what reference_runs_over_threads returns, for a checkout without
+    oracle/_ref.  Dicts with num_iter and nev_conv; the record keeps no eigenvalues."""
+    d = json.loads((ROOT / "tests" / "golden" / "reference_iteration_spread.json").read_text())
+    key = (generator, args, nev, nev_max, nev_init)
+    for r in d["runs"]:
+        if (r["generator"], r["args"], r["nev"], r["nev_max"], r["nev_init"]) == key:
+            return r["by_threads"]
+    raise KeyError(f"no recorded reference run for {key}")
+
+
+def pencil_eigenvalues(pen, k):
+    """The k smallest eigenvalues of A x = lambda B x by shift-invert Lanczos (scipy): the eigenvalues a golden path
+    compares with where the recorded reference runs kept none."""
+    import scipy.sparse.linalg as sla
+    A = pen.A.to_scipy().tocsc()
+    B = None if pen.B is None else pen.B.to_scipy().tocsc()
+    return np.sort(sla.eigsh(A, k=k, M=B, sigma=0.0, which="LM", tol=0)[0])
+
+
 @pytest.fixture(scope="session")
 def golden():
     return json.loads((ROOT / "tests" / "golden" / "gcg_reference.json").read_text())

@@ -75,16 +75,26 @@ def test_petsc_binary(tmp_path):
 
 
 # ---- BASELINE config 1: the reference's mesh file data/cube4.dat ---------------------------------------------
-def test_cube4_fixture_is_the_reference_file():
-    """tests/golden/cube4_mesh.json (made by tests/golden/make_cube4_fixture.py) against the reader run on the
-    reference's own file, where the reference tree is present (this container)."""
-    from pathlib import Path
-    src = Path("/root/reference/data/cube4.dat")
+def test_cube4_fixture_is_the_reference_file(tmp_path):
+    """tests/golden/cube4_mesh.json (made by tests/golden/make_cube4_fixture.py from the reference's data/cube4.dat)
+    holds what that file says -- 125 vertices, exactly the 5^3 lattice of [0,1]^3, 384 tetrahedra over them -- and
+    goes through the ALBERT reader unchanged when written back in the file's format.  The digest pins the vertex
+    and element lists to the ones make_cube4_fixture.py parsed from that file when the fixture was made."""
+    import hashlib
     V, T = P.cube4_mesh()
     assert V.shape == (125, 3) and T.shape == (384, 4)
-    if src.exists():
-        V2, T2 = P.read_albert_mesh(src)
-        assert np.array_equal(V, V2) and np.array_equal(T, T2)
+    q = np.rint(V * 4).astype(np.int64)
+    assert hashlib.sha256(q.tobytes() + T.astype(np.int64).tobytes()).hexdigest() == \
+        "17f73130985d1518b5cdc9ed62f4d6c0769e847b90caaf5d1ecf2117366c0127"
+    assert np.array_equal(q / 4.0, V) and len(np.unique(q, axis=0)) == 125 and q.min() == 0 and q.max() == 4
+    assert T.min() == 0 and T.max() == 124 and all(len(set(t)) == 4 for t in T.tolist())
+    fmt = lambda rows: "\n".join(" ".join(repr(v) for v in r) for r in rows)
+    (tmp_path / "cube4.dat").write_text(
+        "DIM: 3\nDIM_OF_WORLD: 3\n\nnumber of elements: 384\nnumber of vertices: 125\n\n"
+        f"vertex coordinates:\n{fmt(V.tolist())}\n\nelement vertices:\n{fmt(T.tolist())}\n\n"
+        f"element boundaries:\n{fmt(np.zeros_like(T).tolist())}\n")
+    V2, T2 = P.read_albert_mesh(tmp_path / "cube4.dat")
+    assert np.array_equal(V, V2) and np.array_equal(T, T2)
 
 
 def test_cube4_mesh_is_a_conforming_triangulation_of_the_unit_cube():
