@@ -42,7 +42,8 @@ static int bpcg_chunk(const b200_mat *A, const b200_mat *B, long long n,
 	 * vs. launched -- how much a compaction of the active columns could save */
 	const int trace = b200k_opt(B200K_OPT_BPCG_TRACE);
 	long long act_sum = 0, iters_run = 0;
-	for (int it = 0; it < prm->max_iter; ++it) {
+	int it = 0;
+	for (; it < prm->max_iter; ++it) {
 		if (trace) {
 			int c2[2];
 			if (b200k_d2h(c2, st.counters, sizeof(c2))) return 1;
@@ -67,8 +68,8 @@ static int bpcg_chunk(const b200_mat *A, const b200_mat *B, long long n,
 		}
 		if (b200k_bpcg_update_r(n, &st, w, ldw, r, ldr, prm->rate, prm->tol, it)) return 1;
 	}
-	/* the x update of the last iteration that ran */
-	if (b200k_bpcg_update_px(n, &st, r, ldr, p, ldp, x, ldx, prm->max_iter, 1)) return 1;
+	/* the x update of the last iteration that ran; `it`, not max_iter: the trace leaves the loop early */
+	if (b200k_bpcg_update_px(n, &st, r, ldr, p, ldp, x, ldx, it, 1)) return 1;
 	if (trace) fprintf(stderr, "bpcg k=%d: %lld iterations, active column-iterations %lld of %lld (%.0f %%)\n", k, iters_run,
 	                   act_sum, iters_run * k, iters_run ? 100.0 * act_sum / (iters_run * k) : 0.0);
 	if (niter || residual) {

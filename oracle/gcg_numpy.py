@@ -281,10 +281,12 @@ def mgs(x, start_x, end_x, B, prm: OrthParams, orth_self="column"):
 
 
 # ------------------------------------------------------------------------ BlockPCG
-def block_pcg(A, b, x, max_iter, rate, tol, tol_type="abs", shift=0.0, B=None):
+def block_pcg(A, b, x, max_iter, rate, tol, tol_type="abs", shift=0.0, B=None, return_info=False):
     """BlockPCG, reference src/ops_lin_sol.c:140-437 (operator A + shift*B as in
     MatDotMultiVecShift, reference src/ops_eig_sol_gcg.c:63-96).  x is updated in place.
-    Returns (niter, residual norms)."""
+    Returns (niter, residual norms); with return_info also a dict with "stop" (per column, the
+    number of iterations that updated it) and "ratios" (residual / threshold of every comparison
+    behind a stop decision: how close each decision was)."""
     k = b.shape[1]
 
     def op(v):
@@ -299,10 +301,13 @@ def block_pcg(A, b, x, max_iter, rate, tol, tol_type="abs", shift=0.0, B=None):
     init_res = np.sqrt(rho2)
     last_res = init_res.copy()
     unconv = [i for i in range(k) if init_res[i] > tol * norm_b[i]]
+    stop = np.zeros(k, dtype=int)
+    ratios = [init_res[i] / (tol * norm_b[i]) for i in range(k) if tol * norm_b[i] > 0]
     p = np.zeros_like(r)
     rho1 = np.zeros(k)
     niter = 0
     while niter < max_iter and unconv:
+        stop[unconv] += 1
         u = np.array(unconv)
         beta = np.zeros(len(u)) if niter == 0 else rho2[u] / rho1[u]
         p[:, u] = r[:, u] + p[:, u] * beta
@@ -314,8 +319,12 @@ def block_pcg(A, b, x, max_iter, rate, tol, tol_type="abs", shift=0.0, B=None):
         r[:, u] -= w * alpha
         rho2[u] = np.sum(r[:, u] * r[:, u], axis=0)
         last_res[u] = np.sqrt(rho2[u])
+        if return_info:
+            ratios += [last_res[i] / t for i in unconv for t in (rate * init_res[i], tol * norm_b[i]) if t > 0]
         unconv = [i for i in unconv if last_res[i] > rate * init_res[i] and last_res[i] > tol * norm_b[i]]
         niter += 1
+    if return_info:
+        return niter, last_res, {"stop": stop, "ratios": np.array(ratios)}
     return niter, last_res
 
 

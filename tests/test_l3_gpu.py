@@ -1,6 +1,8 @@
 """GPU parity of the fused L3 providers: orthogonalisation (reference test/test_orth.c:21-178
 turned into assertions), BlockPCG (reference test/test_lin_sol.c:58-116) and the projected
 eigen-solve that replaces dsyevx."""
+import ctypes as C
+
 import numpy as np
 import pytest
 
@@ -203,28 +205,34 @@ def test_block_pcg_like_reference_TestMultiLinearSolver(b200, refmod):
 
 @pytest.mark.parametrize("k", [10, 40])
 def test_block_pcg_fused_dot_matches_streaming_dot(b200, k):
-    """The SpMM with diag(p^T A p) in its epilogue (b200_spmm.cu: spmm_dia_ws_kernel<.., DOT>)
-    against the SpMM + streaming dot kernel pair: same iteration count, same iterate up to the
-    rounding of the differently ordered dot products."""
-    import os
+    """The SpMM with diag(p^T A p) in its epilogue (b200_spmm_lat.cu: spmm_lat_kernel<.., DOT>) against the SpMM +
+    streaming dot kernel pair (option no_fused_dot): same iteration count, same iterate up to the rounding of the
+    differently ordered dot products.  The profiler's call counts show that the two arms took different paths."""
     pen = P.p1_fem_kuhn(14)
     n = pen.A.ncols
     A = b200.Mat(pen.A)
+    L = b200.lib()
     rng = np.random.default_rng(11)
     bh = np.asfortranarray(rng.random((n, k)))
     out = []
-    for env in ("", "1"):
-        if env:
-            os.environ["B200_NO_FUSED_DOT"] = env
-        else:
-            os.environ.pop("B200_NO_FUSED_DOT", None)
+    for no_fused in (0, 1):
+        old = C.c_int(0)
+        assert L.b200_option_get(b"no_fused_dot", C.byref(old)) == 0
+        assert L.b200_option_set(b"no_fused_dot", no_fused) == 0
         try:
             X = b200.MultiVec(n, k)
+            b200.prof_enable(True)
             niter, res = b200.block_pcg(A, b200.MultiVec.from_numpy(bh), X, (0, 0), (k, k), max_iter=30, rate=1e-2,
                                         tol=1e-14)
-            out.append((niter, X.numpy()))
+            rep = b200.prof_report()
         finally:
-            os.environ.pop("B200_NO_FUSED_DOT", None)
+            b200.prof_enable(False)
+            L.b200_option_set(b"no_fused_dot", old.value)
+        out.append((niter, X.numpy(), rep["small_dense"]["calls"], rep["bpcg_fused"]["calls"]))
+    # fused: the one-CTA reduction of the SpMM's partial sums in each of the 30 launched steps; streaming: no such
+    # reduction, one more streaming kernel (p^T w) per step instead
+    assert out[0][2] == 30 and out[1][2] == 0, (out[0][2:], out[1][2:])
+    assert out[1][3] == out[0][3] + 30, (out[0][2:], out[1][2:])
     assert out[0][0] == out[1][0]
     assert np.abs(out[0][1] - out[1][1]).max() < 1e-11 * np.abs(out[1][1]).max()
     # and it solves the system: 30 iterations at rate 1e-2 bring the residual down by > 10

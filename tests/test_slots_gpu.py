@@ -62,8 +62,8 @@ def test_device_matrix_build_matches_host_build(b200, name):
     """b200_matbuild.cu (CCS -> CSR slab, symmetry flag, diagonal image, all on the device) against
     the host construction (b200_partition_build + dia_build): the CSR image bit for bit, the CCS
     round trip, and the SpMM result (which goes through the diagonal image where there is one)."""
-    import os
     from gcge_b200 import api
+    L = api.lib()
     if name == "p1":
         M = P.p1_fem_kuhn(11).A
     elif name == "p1_mass":
@@ -87,14 +87,17 @@ def test_device_matrix_build_matches_host_build(b200, name):
         M = P.CCS(30, 20, m.indptr.astype(np.int32), m.indices.astype(np.int32), m.data.astype(np.float64))
     rng = np.random.default_rng(1)
     x = np.asfortranarray(rng.standard_normal((M.ncols, 8)))
-    res = []
-    for host in (False, True):
-        if host:
-            os.environ["B200_HOST_BUILD"] = "1"
+    res, launches = [], []
+    for host in (0, 1):
+        old = C.c_int(0)
+        assert L.b200_option_get(b"host_build", C.byref(old)) == 0
+        assert L.b200_option_set(b"host_build", host) == 0
         try:
+            l0 = L.b200_kernel_launches()
             A = b200.Mat(M)
+            launches.append(L.b200_kernel_launches() - l0)
         finally:
-            os.environ.pop("B200_HOST_BUILD", None)
+            L.b200_option_set(b"host_build", old.value)
         nnz = int(M.j_col[-1])
         rp = np.zeros(M.nrows + 1, np.int32); ci = np.zeros(max(nnz, 1), np.int32); va = np.zeros(max(nnz, 1))
         api._chk(api.lib().b200_mat_local_csr(A.h, ip(rp), ip(ci), dp(va)))
@@ -102,6 +105,10 @@ def test_device_matrix_build_matches_host_build(b200, name):
         api.mat_dot_multivec(A, X, Y, (0, 0), (8, 8))
         res.append((rp, ci[:nnz], va[:nnz], A.to_ccs(), Y.numpy()))
     d, h = res
+    # the device build launches its mb_* kernels (even where it hands over to the host build, as for the long row);
+    # the host build launches none of them
+    print(f"\nmatrix build {name}: kernel launches device {launches[0]}, host {launches[1]}")
+    assert launches[0] > launches[1], launches
     assert np.array_equal(d[0], h[0]) and np.array_equal(d[1], h[1]) and np.array_equal(d[2], h[2])
     for a, b in zip(d[3], h[3]):
         assert np.array_equal(a, b)
