@@ -14,6 +14,12 @@
 // The x update of iteration i is deferred into the p update of iteration i+1: x does not feed back
 // into the iteration, so the iterates are bit-identical to the textbook order (x += alpha p next to
 // r -= alpha w, 6 + 3 streams), and p is read once for both -- 8 streams instead of 9.
+//
+// Jacobi preconditioner (template flag JAC, st.dinv != NULL): z = D^-1 r is never stored.  begin and
+// update_r form it in registers from the r they hold and add r^T z as one more accumulator; update_px
+// forms it again from the r it reads, p = z + beta p.  D^-1 is one double per row shared by the k
+// columns: +8n bytes per launch.  p^T A p is unchanged, so every SpMM path serves as it is.  The JAC =
+// false instantiations are the unpreconditioned kernels unchanged.
 #include "b200_stream.cuh"
 
 constexpr int BPCG_CTAS_MAX = 8;                 // buffers are sized for this many CTAs per SM
@@ -24,7 +30,7 @@ static inline int bpcg_ctas() { const int v = b200_opt(B200_OPT_BPCG_CTAS); retu
 extern "C" int b200k_bpcg_state(int k, b200_bpcg_state *st)
 {
 	const int chunks_max = g_b200.num_sms * BPCG_CTAS_MAX + 8;
-	const size_t dbl = (size_t)9 * k + (size_t)chunks_max * 2 * k;
+	const size_t dbl = (size_t)10 * k + (size_t)chunks_max * 3 * k;
 	const size_t bytes = sizeof(double) * dbl + sizeof(int) * ((size_t)k + 8) + 64;
 	char *base = (char *)b200_scratch(4, bytes);
 	if (!base) return 1;
@@ -32,9 +38,10 @@ extern "C" int b200k_bpcg_state(int k, b200_bpcg_state *st)
 	st->k = k;
 	st->norm_b = d; st->rho1 = d + k; st->rho2 = d + 2 * k; st->ptw = d + 3 * k;
 	st->init_res = d + 4 * k; st->last_res = d + 5 * k;
-	st->totals = d + 6 * k;                       /* 2k: per-column sums of the current reduction */
-	st->alpha = d + 8 * k;                        /* k: step length of the x update still to be applied */
-	st->partials = d + 9 * k;
+	st->totals = d + 6 * k;                       /* 3k: per-column sums of the current reduction */
+	st->alpha = d + 9 * k;                        /* k: step length of the x update still to be applied */
+	st->partials = d + 10 * k;                    /* chunks x 3 accumulators x k */
+	st->dinv = nullptr;
 	int *ip = (int *)(d + dbl);
 	st->active = ip; st->counters = ip + k; st->tickets = (unsigned *)(ip + k + 4);
 	B200_CUDA(cudaMemsetAsync(st->counters, 0, sizeof(int) * 8, g_b200.stream));
@@ -47,6 +54,8 @@ extern "C" int b200k_bpcg_state(int k, b200_bpcg_state *st)
 // MPI_Allreduce at src/ops_lin_sol.c:317,365) and then this runs as a one-CTA kernel -- every
 // rank computes the same alpha / beta / masks from the same bits.
 //   phase 0: after r = b - A x     phase 1: after p^T w     phase 2: after r -= alpha w
+// totals: phase 0 [r^T r | b^T b | r^T z], phase 2 [r^T r | r^T z]; rho is r^T z with JAC, else r^T r
+template <bool JAC>
 __device__ __forceinline__ void bpcg_scalar_phase(int phase, int k, const b200_bpcg_state &st, double tol, int rel,
                                                   double rate)
 {
@@ -56,9 +65,10 @@ __device__ __forceinline__ void bpcg_scalar_phase(int phase, int k, const b200_b
 	for (int c = threadIdx.x; c < k; c += blockDim.x) {
 		if (phase == 0) {
 			const double rr = st.totals[c], bb = st.totals[k + c];
+			const double rho = JAC ? st.totals[2 * k + c] : rr;
 			const double nb = rel ? sqrt(bb) : 1.0;
 			const double res = sqrt(rr);
-			st.norm_b[c] = nb; st.rho2[c] = rr; st.rho1[c] = rr;
+			st.norm_b[c] = nb; st.rho2[c] = rho; st.rho1[c] = rho;
 			st.init_res[c] = res; st.last_res[c] = res;
 			const int act = (res > tol * nb) ? 1 : 0;      // reference src/ops_lin_sol.c:239-247
 			st.active[c] = act;
@@ -68,7 +78,7 @@ __device__ __forceinline__ void bpcg_scalar_phase(int phase, int k, const b200_b
 		} else if (st.active[c]) {
 			const double rr = st.totals[c];
 			st.rho1[c] = st.rho2[c];
-			st.rho2[c] = rr;
+			st.rho2[c] = JAC ? st.totals[k + c] : rr;
 			const double res = sqrt(rr);
 			st.last_res[c] = res;
 			// reference src/ops_lin_sol.c:383-394: stay active while res > rate*res0 AND res > tol*||b||
@@ -99,15 +109,16 @@ __device__ __forceinline__ void bpcg_store_totals(int k, const b200_bpcg_state &
 	__syncthreads();
 }
 
+template <bool JAC>
 __global__ void bpcg_finish_kernel(int phase, int k, b200_bpcg_state st, double tol, int rel, double rate)
 {
 	if (phase != 0 && st.counters[0] == 0) return;
-	bpcg_scalar_phase(phase, k, st, tol, rel, rate);
+	bpcg_scalar_phase<JAC>(phase, k, st, tol, rel, rate);
 }
 
 // ---------------------------------------------------------------------------- begin
-// r <- b - r ; acc0 = r.r ; acc1 = b.b (rel only)
-template <int VEC>
+// r <- b - r ; acc0 = r.r ; acc1 = b.b (rel only) ; JAC: acc2 = r.z, z = D^-1 r
+template <int VEC, bool JAC>
 __global__ void __launch_bounds__(ST_THREADS)
 bpcg_begin_kernel(long long n, int k, StreamGeom g, const double *__restrict__ b, int ldb, double *__restrict__ r, int ldr,
                   double tol, int rel, int defer, b200_bpcg_state st, B200ArCtx ar)
@@ -115,16 +126,23 @@ bpcg_begin_kernel(long long n, int k, StreamGeom g, const double *__restrict__ b
 	const StreamThread t = stream_thread<VEC>(g);
 	const long long r_begin = (long long)blockIdx.x * g.rows_per_chunk;
 	long long r_end = r_begin + g.rows_per_chunk; if (r_end > n) r_end = n;
-	double acc[2][VEC];
+	constexpr int NACC = JAC ? 3 : 2;
+	double acc[NACC][VEC];
 #pragma unroll
-	for (int i = 0; i < VEC; ++i) { acc[0][i] = 0.0; acc[1][i] = 0.0; }
+	for (int a = 0; a < NACC; ++a)
+#pragma unroll
+		for (int i = 0; i < VEC; ++i) acc[a][i] = 0.0;
 	if (t.active) {
 		for (long long row0 = r_begin + t.rl; row0 < r_end; row0 += (long long)ST_UNROLL * g.rp) {
 			StV<VEC> bv[ST_UNROLL], rv[ST_UNROLL];
+			double dv[ST_UNROLL];
 #pragma unroll
 			for (int u = 0; u < ST_UNROLL; ++u) {
 				const long long row = row0 + (long long)u * g.rp;
-				if (row < r_end) { bv[u] = st_ld<VEC>(b + (size_t)row * ldb + t.c); rv[u] = st_ld<VEC>(r + (size_t)row * ldr + t.c); }
+				if (row < r_end) {
+					bv[u] = st_ld<VEC>(b + (size_t)row * ldb + t.c); rv[u] = st_ld<VEC>(r + (size_t)row * ldr + t.c);
+					if constexpr (JAC) dv[u] = st.dinv[row];
+				}
 			}
 #pragma unroll
 			for (int u = 0; u < ST_UNROLL; ++u) {
@@ -136,16 +154,17 @@ bpcg_begin_kernel(long long n, int k, StreamGeom g, const double *__restrict__ b
 						rv[u].v[i] = x;
 						acc[0][i] = fma(x, x, acc[0][i]);
 						acc[1][i] = fma(bv[u].v[i], bv[u].v[i], acc[1][i]);
+						if constexpr (JAC) acc[NACC - 1][i] = fma(x, dv[u] * x, acc[NACC - 1][i]);
 					}
 					st_st<VEC>(r + (size_t)row * ldr + t.c, rv[u]);
 				}
 			}
 		}
 	}
-	if (!stream_reduce_and_elect<VEC, 2>(acc, k, g, t, st.partials, st.tickets)) return;
-	bpcg_store_totals<2>(k, st);
-	if (ar.nranks > 1) stream_allreduce_cta(ar, st.totals, 2 * k);
-	if (!defer) bpcg_scalar_phase(0, k, st, tol, rel, 0.0);
+	if (!stream_reduce_and_elect<VEC, NACC>(acc, k, g, t, st.partials, st.tickets)) return;
+	bpcg_store_totals<NACC>(k, st);
+	if (ar.nranks > 1) stream_allreduce_cta(ar, st.totals, NACC * k);
+	if (!defer) bpcg_scalar_phase<JAC>(0, k, st, tol, rel, 0.0);
 }
 
 // ------------------------------------------------------------------------------ ptw
@@ -192,13 +211,14 @@ bpcg_ptw_kernel(long long n, int k, StreamGeom g, const double *p, int ldp, doub
 	if (!stream_reduce_and_elect<VEC, 1>(acc, k, g, t, st.partials, st.tickets)) return;
 	bpcg_store_totals<1>(k, st);
 	if (ar.nranks > 1) stream_allreduce_cta(ar, st.totals, k);
-	if (!defer) bpcg_scalar_phase(1, k, st, 0.0, 0, 0.0);
+	if (!defer) bpcg_scalar_phase<false>(1, k, st, 0.0, 0, 0.0);
 }
 
 // ------------------------------------------------------------------------- update_r
-// alpha = rho2/ptw ; r -= alpha w ; rho1 = rho2 ; rho2 = diag(r^T r) ; stop test.  alpha is left in
-// st.alpha for the deferred x update; counters[2] = it + 1 says which iteration it belongs to.
-template <int VEC>
+// alpha = rho2/ptw ; r -= alpha w ; rho1 = rho2 ; rho2 = diag(r^T r) (JAC: diag(r^T z)) ; stop test on
+// sqrt(r^T r).  alpha is left in st.alpha for the deferred x update; counters[2] = it + 1 says which
+// iteration it belongs to.
+template <int VEC, bool JAC>
 __global__ void __launch_bounds__(ST_THREADS)
 bpcg_update_r_kernel(long long n, int k, StreamGeom g, const double *__restrict__ w, int ldw, double *__restrict__ r, int ldr,
                      double rate, double tol, int it, int defer, b200_bpcg_state st, B200ArCtx ar)
@@ -207,11 +227,13 @@ bpcg_update_r_kernel(long long n, int k, StreamGeom g, const double *__restrict_
 	const StreamThread t = stream_thread<VEC>(g);
 	const long long r_begin = (long long)blockIdx.x * g.rows_per_chunk;
 	long long r_end = r_begin + g.rows_per_chunk; if (r_end > n) r_end = n;
-	double acc[1][VEC], alpha[VEC];
+	constexpr int NACC = JAC ? 2 : 1;
+	double acc[NACC][VEC], alpha[VEC];
 	bool act[VEC]; bool any = false;
 #pragma unroll
 	for (int i = 0; i < VEC; ++i) {
-		acc[0][i] = 0.0;
+#pragma unroll
+		for (int a = 0; a < NACC; ++a) acc[a][i] = 0.0;
 		act[i] = t.active && st.active[t.c + i];
 		alpha[i] = act[i] ? st.rho2[t.c + i] / st.ptw[t.c + i] : 0.0;       // reference src/ops_lin_sol.c:328
 		any = any || act[i];
@@ -224,12 +246,14 @@ bpcg_update_r_kernel(long long n, int k, StreamGeom g, const double *__restrict_
 	if (any) {
 		for (long long row0 = r_begin + t.rl; row0 < r_end; row0 += (long long)ST_UNROLL * g.rp) {
 			StV<VEC> wv[ST_UNROLL], rv[ST_UNROLL];
+			double dv[ST_UNROLL];
 #pragma unroll
 			for (int u = 0; u < ST_UNROLL; ++u) {
 				const long long row = row0 + (long long)u * g.rp;
 				if (row < r_end) {
 					wv[u] = st_ld<VEC>(w + (size_t)row * ldw + t.c);
 					rv[u] = st_ld<VEC>(r + (size_t)row * ldr + t.c);
+					if constexpr (JAC) dv[u] = st.dinv[row];
 				}
 			}
 #pragma unroll
@@ -242,6 +266,7 @@ bpcg_update_r_kernel(long long n, int k, StreamGeom g, const double *__restrict_
 							const double nr = fma(-alpha[i], wv[u].v[i], rv[u].v[i]);
 							rv[u].v[i] = nr;
 							acc[0][i] = fma(nr, nr, acc[0][i]);
+							if constexpr (JAC) acc[NACC - 1][i] = fma(nr, dv[u] * nr, acc[NACC - 1][i]);
 						}
 					}
 					st_st<VEC>(r + (size_t)row * ldr + t.c, rv[u]);
@@ -249,17 +274,17 @@ bpcg_update_r_kernel(long long n, int k, StreamGeom g, const double *__restrict_
 			}
 		}
 	}
-	if (!stream_reduce_and_elect<VEC, 1>(acc, k, g, t, st.partials, st.tickets)) return;
-	bpcg_store_totals<1>(k, st);
-	if (ar.nranks > 1) stream_allreduce_cta(ar, st.totals, k);
-	if (!defer) bpcg_scalar_phase(2, k, st, tol, 0, rate);
+	if (!stream_reduce_and_elect<VEC, NACC>(acc, k, g, t, st.partials, st.tickets)) return;
+	bpcg_store_totals<NACC>(k, st);
+	if (ar.nranks > 1) stream_allreduce_cta(ar, st.totals, NACC * k);
+	if (!defer) bpcg_scalar_phase<JAC>(2, k, st, tol, 0, rate);
 }
 
 // ------------------------------------------------------------------------ update_px
 // x += alpha p for the step length left by update_r of iteration `expect - 1` (if any), then
-// p = r + (rho2/rho1) p on the columns still active (reference src/ops_lin_sol.c:271-284, :330-340).
-// flush: only the x update (after the last iteration).
-template <int VEC>
+// p = r + (rho2/rho1) p on the columns still active (reference src/ops_lin_sol.c:271-284, :330-340);
+// JAC: p = D^-1 r + (rho2/rho1) p.  flush: only the x update (after the last iteration).
+template <int VEC, bool JAC>
 __global__ void __launch_bounds__(ST_THREADS)
 bpcg_update_px_kernel(long long n, int k, StreamGeom g, const double *__restrict__ r, int ldr, double *__restrict__ p,
                       int ldp, double *__restrict__ x, int ldx, int first, int expect, int flush, b200_bpcg_state st)
@@ -283,11 +308,13 @@ bpcg_update_px_kernel(long long n, int k, StreamGeom g, const double *__restrict
 	long long r_end = r_begin + g.rows_per_chunk; if (r_end > n) r_end = n;
 	for (long long row0 = r_begin + t.rl; row0 < r_end; row0 += (long long)ST_UNROLL * g.rp) {
 		StV<VEC> rv[ST_UNROLL], pv[ST_UNROLL], xv[ST_UNROLL];
+		double dv[ST_UNROLL];
 #pragma unroll
 		for (int u = 0; u < ST_UNROLL; ++u) {
 			const long long row = row0 + (long long)u * g.rp;
 			if (row < r_end) {
 				if (any_p) rv[u] = st_ld<VEC>(r + (size_t)row * ldr + t.c);
+				if constexpr (JAC) { if (any_p) dv[u] = st.dinv[row]; }
 				pv[u] = st_ld<VEC>(p + (size_t)row * ldp + t.c);
 				if (any_x) xv[u] = st_ld<VEC>(x + (size_t)row * ldx + t.c);
 			}
@@ -303,6 +330,10 @@ bpcg_update_px_kernel(long long n, int k, StreamGeom g, const double *__restrict
 					st_st<VEC>(x + (size_t)row * ldx + t.c, xv[u]);
 				}
 				if (any_p) {
+					if constexpr (JAC) {
+#pragma unroll
+						for (int i = 0; i < VEC; ++i) rv[u].v[i] *= dv[u];
+					}
 #pragma unroll
 					for (int i = 0; i < VEC; ++i)
 						if (act[i]) pv[u].v[i] = first ? rv[u].v[i] : fma(beta[i], pv[u].v[i], rv[u].v[i]);
@@ -326,7 +357,8 @@ static B200ArCtx bpcg_ar(int count)
 static int bpcg_finish(int phase, int nacc, const b200_bpcg_state *st, double tol, int rel, double rate)
 {
 	if (b200k_allreduce_sum(st->totals, (size_t)nacc * st->k)) return 1;
-	bpcg_finish_kernel<<<1, 128, 0, g_b200.stream>>>(phase, st->k, *st, tol, rel, rate);
+	if (st->dinv && phase != 1) bpcg_finish_kernel<true><<<1, 128, 0, g_b200.stream>>>(phase, st->k, *st, tol, rel, rate);
+	else bpcg_finish_kernel<false><<<1, 128, 0, g_b200.stream>>>(phase, st->k, *st, tol, rel, rate);
 	B200_KERNEL_CHECK();
 	return 0;
 }
@@ -335,14 +367,19 @@ extern "C" int b200k_bpcg_begin(long long n, const b200_bpcg_state *st, const do
                                 double *r, int ldr, double tol, int rel)
 {
 	const int k = st->k;
-	const B200ArCtx ar = bpcg_ar(2 * k);
+	const bool jac = st->dinv != nullptr;
+	const int nacc = jac ? 3 : 2;
+	const B200ArCtx ar = bpcg_ar(nacc * k);
 	const int defer = (b200_multi() && ar.nranks == 0) ? 1 : 0;
 	B200_CHECK(k >= 1 && k <= 128, "BlockPCG: %d columns (1..128 supported per block)", k);
-	B200Prof prof(B200_PROF_BPCG, 24.0 * n * k, 5.0 * n * k);
+	B200Prof prof(B200_PROF_BPCG, 24.0 * n * k + (jac ? 8.0 * n : 0.0), (jac ? 8.0 : 5.0) * n * k);
 	const StreamGeom g = stream_geometry(n, k, stream_aligned16(b, ldb) && stream_aligned16(r, ldr), BPCG_CTAS_PER_SM);
-	ST_DISPATCH_VEC(g, (bpcg_begin_kernel<VEC><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, b, ldb, r, ldr, tol, rel, defer, *st, ar)));
+	if (jac)
+		ST_DISPATCH_VEC(g, (bpcg_begin_kernel<VEC, true><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, b, ldb, r, ldr, tol, rel, defer, *st, ar)));
+	else
+		ST_DISPATCH_VEC(g, (bpcg_begin_kernel<VEC, false><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, b, ldb, r, ldr, tol, rel, defer, *st, ar)));
 	B200_KERNEL_CHECK();
-	if (defer) return bpcg_finish(0, 2, st, tol, rel, 0.0);
+	if (defer) return bpcg_finish(0, nacc, st, tol, rel, 0.0);
 	return 0;
 }
 
@@ -373,7 +410,7 @@ bpcg_ptw_parts_kernel(int nparts, int k, int defer, b200_bpcg_state st, B200ArCt
 	}
 	__syncthreads();
 	if (ar.nranks > 1) stream_allreduce_cta(ar, st.totals, k);
-	if (!defer) bpcg_scalar_phase(1, k, st, 0.0, 0, 0.0);
+	if (!defer) bpcg_scalar_phase<false>(1, k, st, 0.0, 0, 0.0);
 }
 
 int b200k_spmm_dot(const b200_mat *M, const double *x, int ldx, double *y, int ldy, int k, const int *gate,
@@ -410,13 +447,18 @@ extern "C" int b200k_bpcg_update_r(long long n, const b200_bpcg_state *st, const
                                    double rate, double tol, int it)
 {
 	const int k = st->k;
-	const B200ArCtx ar = bpcg_ar(k);
+	const bool jac = st->dinv != nullptr;
+	const int nacc = jac ? 2 : 1;
+	const B200ArCtx ar = bpcg_ar(nacc * k);
 	const int defer = (b200_multi() && ar.nranks == 0) ? 1 : 0;
-	B200Prof prof(B200_PROF_BPCG, 24.0 * n * k, 4.0 * n * k);
+	B200Prof prof(B200_PROF_BPCG, 24.0 * n * k + (jac ? 8.0 * n : 0.0), (jac ? 7.0 : 4.0) * n * k);
 	const StreamGeom g = stream_geometry(n, k, stream_aligned16(w, ldw) && stream_aligned16(r, ldr), BPCG_CTAS_PER_SM);
-	ST_DISPATCH_VEC(g, (bpcg_update_r_kernel<VEC><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, w, ldw, r, ldr, rate, tol, it, defer, *st, ar)));
+	if (jac)
+		ST_DISPATCH_VEC(g, (bpcg_update_r_kernel<VEC, true><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, w, ldw, r, ldr, rate, tol, it, defer, *st, ar)));
+	else
+		ST_DISPATCH_VEC(g, (bpcg_update_r_kernel<VEC, false><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, w, ldw, r, ldr, rate, tol, it, defer, *st, ar)));
 	B200_KERNEL_CHECK();
-	if (defer) return bpcg_finish(2, 1, st, tol, 0, rate);
+	if (defer) return bpcg_finish(2, nacc, st, tol, 0, rate);
 	return 0;
 }
 
@@ -426,11 +468,89 @@ extern "C" int b200k_bpcg_update_px(long long n, const b200_bpcg_state *st, cons
                                     double *x, int ldx, int it, int flush)
 {
 	const int k = st->k;
-	B200Prof prof(B200_PROF_BPCG, (flush ? 24.0 : (it == 0 ? 24.0 : 40.0)) * n * k, 4.0 * n * k);
+	const bool jac = st->dinv != nullptr && !flush;       // the flush updates x only
+	B200Prof prof(B200_PROF_BPCG, (flush ? 24.0 : (it == 0 ? 24.0 : 40.0)) * n * k + (jac ? 8.0 * n : 0.0),
+	              (jac ? 5.0 : 4.0) * n * k);
 	const StreamGeom g = stream_geometry(n, k, stream_aligned16(r, ldr) && stream_aligned16(p, ldp) && stream_aligned16(x, ldx),
 	                                     BPCG_CTAS_PER_SM);
-	ST_DISPATCH_VEC(g, (bpcg_update_px_kernel<VEC><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, r, ldr, p, ldp, x, ldx,
-	                                                                                         it == 0, it, flush, *st)));
+	if (jac)
+		ST_DISPATCH_VEC(g, (bpcg_update_px_kernel<VEC, true><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, r, ldr, p, ldp, x, ldx,
+		                                                                                               it == 0, it, flush, *st)));
+	else
+		ST_DISPATCH_VEC(g, (bpcg_update_px_kernel<VEC, false><<<g.chunks, ST_THREADS, 0, g_b200.stream>>>(n, k, g, r, ldr, p, ldp, x, ldx,
+		                                                                                                it == 0, it, flush, *st)));
 	B200_KERNEL_CHECK();
+	return 0;
+}
+
+// ------------------------------------------------------------------------- Jacobi diagonal
+// the entry (row, row) of a CSR; found = false when it is not stored.  On a row slab the diagonal of local row r has
+// local column r in both halo layouts (b200_dev.h, struct b200_mat_).  A linear scan: the remapped columns of a slab
+// with a scattered halo are not ascending, and the rows are short.
+__device__ __forceinline__ double csr_diag(const int *__restrict__ rp, const int *__restrict__ ci, const double *__restrict__ va,
+                                           int row, bool &found)
+{
+	const int e1 = rp[row + 1];
+	for (int e = rp[row]; e < e1; ++e)
+		if (ci[e] == row) { found = true; return va[e]; }
+	found = false;
+	return 0.0;
+}
+
+// dinv[row] = 1 / (a_rr + shift b_rr)  (bmode 1),  1 / (a_rr + shift)  (bmode 2),  1 / a_rr  (bmode 0).
+// bad[0] counts the rows without a stored diagonal or with one that is not > 0 (NaN included); ibad[0] = the smallest
+// such row (memset to 0x7f7f7f7f before).
+__global__ void __launch_bounds__(256)
+bpcg_jacobi_diag_kernel(int n, const int *__restrict__ arp, const int *__restrict__ aci, const double *__restrict__ ava,
+                        const int *__restrict__ brp, const int *__restrict__ bci, const double *__restrict__ bva,
+                        double shift, int bmode, double *__restrict__ dinv, double *__restrict__ bad, int *__restrict__ ibad)
+{
+	for (int row = blockIdx.x * blockDim.x + threadIdx.x; row < n; row += gridDim.x * blockDim.x) {
+		bool fa = false, fb = true;
+		double d = csr_diag(arp, aci, ava, row, fa);
+		if (bmode == 1) d += shift * csr_diag(brp, bci, bva, row, fb);
+		else if (bmode == 2) d += shift;
+		if (!fa || !fb || !(d > 0.0)) {
+			atomicAdd(bad, 1.0);
+			atomicMin(ibad, row);
+			d = 1.0;                      // the solve does not run; keep the buffer finite
+		}
+		dinv[row] = 1.0 / d;
+	}
+}
+
+extern "C" int b200k_bpcg_jacobi(const b200_mat *A, const b200_mat *B, double shift, const double **dinv_dev)
+{
+	const int n = A->nrows;
+	B200_CHECK(A->rp && A->ci && A->va, "BlockPCG Jacobi: the matrix has no device CSR image");
+	const int bmode = (shift == 0.0) ? 0 : (B ? 1 : 2);
+	if (bmode == 1) B200_CHECK(B->nrows == n && B->rp && B->ci && B->va, "BlockPCG Jacobi: B does not match A's rows");
+	char *base = (char *)b200_scratch(10, sizeof(double) * ((size_t)n + 4) + 64);
+	if (!base) return 1;
+	double *dinv = (double *)base, *bad = dinv + n;
+	int *ibad = (int *)(bad + 2);
+	B200_CUDA(cudaMemsetAsync(bad, 0, sizeof(double), g_b200.stream));
+	B200_CUDA(cudaMemsetAsync(ibad, 0x7f, sizeof(int), g_b200.stream));
+	{
+		B200Prof prof(B200_PROF_BPCG, 4.0 * n + 12.0 * A->nnz + (bmode == 1 ? 4.0 * n + 12.0 * B->nnz : 0.0) + 8.0 * n,
+		              (bmode == 1 ? 3.0 : 2.0) * n);
+		const int blocks = n > 0 ? b200_ceil_div(n, 256) : 1;
+		bpcg_jacobi_diag_kernel<<<blocks < 65535 * 16 ? blocks : 65535 * 16, 256, 0, g_b200.stream>>>(
+		    n, A->rp, A->ci, A->va, bmode == 1 ? B->rp : nullptr, bmode == 1 ? B->ci : nullptr, bmode == 1 ? B->va : nullptr,
+		    shift, bmode, dinv, bad, ibad);
+		B200_KERNEL_CHECK();
+	}
+	// every rank has to take the same branch: the count of bad rows is summed over the ranks
+	if (b200_multi() && b200k_allreduce_sum(bad, 1)) return 1;
+	double nbad = 0.0; int first = 0;
+	if (b200k_d2h(&nbad, bad, sizeof(double)) || b200k_d2h(&first, ibad, sizeof(int))) return 1;
+	if (nbad != 0.0) {
+		if (first < n)
+			return b200_fail("BlockPCG Jacobi: %.0f rows of A + shift*B (shift %g) have no diagonal entry or one <= 0 "
+			                 "(first: row %lld)", nbad, shift, (long long)A->row0 + first);
+		return b200_fail("BlockPCG Jacobi: %.0f rows of A + shift*B (shift %g) have no diagonal entry or one <= 0 "
+		                 "(on another rank)", nbad, shift);
+	}
+	*dinv_dev = dinv;
 	return 0;
 }

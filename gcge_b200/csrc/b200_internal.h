@@ -19,9 +19,10 @@ struct b200_ctx {
 	// growable device scratch: [0] reduction partials, [1] coefficient staging,
 	// [2] host<->device column-major staging, [3] small results
 	// [4] BlockPCG state, [5] Jacobi work, [6] halo send buffer, [7] halo receive buffer,
-	// [8] contiguous Gram block for the allreduce, [9] the GCG driver's small device arrays
-	void *scratch[10];
-	size_t scratch_bytes[10];
+	// [8] contiguous Gram block for the allreduce, [9] the GCG driver's small device arrays,
+	// [10] BlockPCG's Jacobi preconditioner D^-1 and its diagonal check
+	void *scratch[11];
+	size_t scratch_bytes[11];
 	// pinned host staging for small results / coefficients
 	void *pinned[2];
 	size_t pinned_bytes[2];

@@ -105,7 +105,7 @@ extern "C" void b200_finalize(void)
 	if (g_b200.pending) b200k_pending_flush();
 	cudaStreamSynchronize(g_b200.stream);
 	b200_gcg_free_cache();
-	for (int i = 0; i < 10; ++i) {
+	for (int i = 0; i < 11; ++i) {
 		if (g_b200.scratch[i]) cudaFree(g_b200.scratch[i]);
 		g_b200.scratch[i] = nullptr; g_b200.scratch_bytes[i] = 0;
 	}

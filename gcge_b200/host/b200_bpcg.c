@@ -10,6 +10,10 @@
  * stay in HBM, and every launch returns at once when no column is active any more, so the
  * host never reads anything back inside the loop.  Converged columns are frozen exactly as
  * in the reference (their x, r, p are no longer updated).
+ *
+ * pc = 1 (b200_block_pcg_pc): point Jacobi, D = diag(A + shift B).  D^-1 is formed once per call by one
+ * kernel over the device CSR (the only synchronisation it adds: a bad diagonal fails the call before
+ * anything is written), and z = D^-1 r lives in registers of the streaming kernels only.
  */
 #include <stdlib.h>
 #include <string.h>
@@ -21,11 +25,12 @@
 
 static int bpcg_chunk(const b200_mat *A, const b200_mat *B, long long n,
                       double *b, int ldb, double *x, int ldx, int k, const b200_bpcg_params *prm,
-                      double *r, int ldr, double *p, int ldp, double *w, int ldw,
+                      double *r, int ldr, double *p, int ldp, double *w, int ldw, const double *dinv,
                       int *niter, double *residual)
 {
 	b200_bpcg_state st;
 	if (b200k_bpcg_state(k, &st)) return 1;
+	st.dinv = dinv;
 	const double shift = prm->shift;
 	/* r = (A + shift B) x, then r = b - r and the initial masks */
 	if (b200k_spmm(A, 0, x, ldx, r, ldr, k, NULL)) return 1;
@@ -84,12 +89,13 @@ static int bpcg_chunk(const b200_mat *A, const b200_mat *B, long long n,
 	return 0;
 }
 
-int b200_block_pcg(const b200_mat *A, const b200_mat *B, b200_mv *b, b200_mv *x,
-                   const int *start, const int *end, const b200_bpcg_params *prm,
-                   b200_mv *ws_r, b200_mv *ws_p, b200_mv *ws_w, int *niter, double *residual)
+int b200_block_pcg_pc(const b200_mat *A, const b200_mat *B, b200_mv *b, b200_mv *x,
+                      const int *start, const int *end, const b200_bpcg_params *prm, int pc,
+                      b200_mv *ws_r, b200_mv *ws_p, b200_mv *ws_w, int *niter, double *residual)
 {
 	if (!A || !b || !x || !start || !end || !prm || !ws_r || !ws_p || !ws_w)
 		return b200_fail("b200_block_pcg: bad arguments");
+	if (pc != 0 && pc != 1) return b200_fail("b200_block_pcg: preconditioner %d (0 none, 1 Jacobi)", pc);
 	if (b200k_pending_flush()) return 1;
 	const int k = end[0] - start[0];
 	if (k != end[1] - start[1]) return b200_fail("b200_block_pcg: column counts differ");
@@ -108,11 +114,20 @@ int b200_block_pcg(const b200_mat *A, const b200_mat *B, b200_mv *b, b200_mv *x,
 	if (ws_w->ncols < wk) wk = ws_w->ncols;
 	if (wk > BPCG_MAX_K) wk = BPCG_MAX_K;
 	if (wk < 1) return b200_fail("b200_block_pcg: workspaces have no columns");
+	const double *dinv = NULL;
+	if (pc == 1 && b200k_bpcg_jacobi(A, B, prm->shift, &dinv)) return 1;      /* D^-1 of the whole call, before x is touched */
 	for (int c0 = 0; c0 < k; c0 += wk) {
 		const int kc = (k - c0 < wk) ? k - c0 : wk;
 		if (bpcg_chunk(A, B, n, b->d + start[0] + c0, b->ld, x->d + start[1] + c0, x->ld, kc, prm,
-		               ws_r->d, ws_r->ld, ws_p->d, ws_p->ld, ws_w->d, ws_w->ld, niter, residual))
+		               ws_r->d, ws_r->ld, ws_p->d, ws_p->ld, ws_w->d, ws_w->ld, dinv, niter, residual))
 			return 1;
 	}
 	return 0;
+}
+
+int b200_block_pcg(const b200_mat *A, const b200_mat *B, b200_mv *b, b200_mv *x,
+                   const int *start, const int *end, const b200_bpcg_params *prm,
+                   b200_mv *ws_r, b200_mv *ws_p, b200_mv *ws_w, int *niter, double *residual)
+{
+	return b200_block_pcg_pc(A, B, b, x, start, end, prm, 0, ws_r, ws_p, ws_w, niter, residual);
 }

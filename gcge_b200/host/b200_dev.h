@@ -160,16 +160,23 @@ typedef struct b200_bpcg_state_ {
 	double *norm_b, *rho1, *rho2, *ptw, *init_res, *last_res;   /* k doubles each (device) */
 	int *active;        /* k ints (device): 1 while the column is unconverged */
 	int *counters;      /* [0] number of active columns, [1] iterations done, [2] 1 + iteration of the pending alpha (device) */
-	double *totals;     /* 2k doubles: per-column sums of the current reduction (allreduced across ranks) */
+	double *totals;     /* 3k doubles: per-column sums of the current reduction (allreduced across ranks) */
 	double *alpha;      /* k doubles: step length of the x update deferred into the next p update */
 	double *partials;   /* reduction scratch */
 	unsigned *tickets;  /* last-block election counters */
+	const double *dinv; /* n doubles (device): Jacobi preconditioner D^-1, NULL: none (b200k_bpcg_state leaves it NULL) */
 } b200_bpcg_state;
 int b200k_bpcg_state(int k, b200_bpcg_state *st);               /* carve state out of scratch */
+/* Jacobi preconditioner of A + shift B (B NULL: A + shift I): *dinv_dev = 1 / diagonal, one double per local row, in a
+ * scratch slot of its own.  Reads the device CSR; fails (synchronises once) when a row has no diagonal entry or a
+ * diagonal <= 0, on any rank. */
+int b200k_bpcg_jacobi(const b200_mat *A, const b200_mat *B, double shift, const double **dinv_dev);
 /* several ranks: 0, or an error if an in-kernel allreduce timed out since the communicator was made (synchronises) */
 int b200k_ar_check(void);
 /* r = b - r (r holds A x on entry); rho2 = diag(r^T r); norm_b = 1 or ||b||; then decide the
- * initial active set: init_res > tol*norm_b (reference src/ops_lin_sol.c:221-247) */
+ * initial active set: init_res > tol*norm_b (reference src/ops_lin_sol.c:221-247).
+ * With st->dinv set (Jacobi), here and in update_r / update_px: z = D^-1 r is formed in registers, rho = diag(r^T z)
+ * drives alpha and beta, p = z + beta p; the residual norms and the stop test stay on sqrt(r^T r). */
 int b200k_bpcg_begin(long long n, const b200_bpcg_state *st, const double *b, int ldb,
                      double *r, int ldr, double tol, int rel);
 /* w += shift * z (optional), ptw = diag(p^T w) */

@@ -281,7 +281,7 @@ static int compute_w(gcg_t *g, const int *offset)
 	bp.tol_type = p->compW_cg_tol_type; bp.shift = sigma;
 	int s[2], e[2];
 	s[0] = b0; e[0] = b0 + acc; s[1] = 0; e[1] = acc;
-	TRY(b200_block_pcg(g->A, g->B, g->ritz, g->xw, s, e, &bp, g->ws[0], g->ws[1], g->ws[2], NULL, NULL));
+	TRY(b200_block_pcg_pc(g->A, g->B, g->ritz, g->xw, s, e, &bp, p->compW_cg_pc, g->ws[0], g->ws[1], g->ws[2], NULL, NULL));
 	/* W block of [X P W] <- the solutions (one pass; the 30 CG steps had x to themselves) */
 	TRY(b200k_axpby(g->n, acc, 1.0, g->xw->d, g->xw->ld, 0.0, g->V->d + g->startW, g->V->ld));
 	double t2 = tick(g);
@@ -349,7 +349,7 @@ static int compute_w12(gcg_t *g, const int *offset)
 		bp.tol_type = p->compW_cg_tol_type; bp.shift = sigma;
 		int s[2], e[2];
 		s[0] = b0; e[0] = b0 + acc; s[1] = g->startW + pass * acc; e[1] = s[1] + acc;
-		if (acc > 0) TRY(b200_block_pcg(g->A, g->B, g->ritz, g->V, s, e, &bp, g->ws[0], g->ws[1], g->ws[2], NULL, NULL));
+		if (acc > 0) TRY(b200_block_pcg_pc(g->A, g->B, g->ritz, g->V, s, e, &bp, p->compW_cg_pc, g->ws[0], g->ws[1], g->ws[2], NULL, NULL));
 		g->st.linsol += tick(g) - t1;
 	}
 	g->endW = g->startW + 2 * acc;
@@ -380,6 +380,7 @@ void b200_gcg_default_params(int nevConv, b200_gcg_params *p)
 	p->compRR_tol = 2 * DBL_EPSILON;
 	p->compW_cg_order = 1;
 	p->verbose = 0;
+	p->compW_cg_pc = 0;
 }
 
 /* The second [X | P | W] buffer is kept between solves (a solver object would own it; the reference's

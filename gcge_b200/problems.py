@@ -200,6 +200,55 @@ def laplace3d_7pt_eigenvalues(m: int, k: int) -> np.ndarray:
     return np.sort(vals)[:k]
 
 
+def diffusion7_var(m: int, coef: str = "lognormal", seed: int = 0, sigma: float = 2.0, mass: bool = False) -> Pencil:
+    """-div(kappa grad u) on an m**3 cell-centred grid, 7-point, harmonic averages of kappa on the faces, Dirichlet
+    faces (2 kappa each), grid spacing 1: heterogeneous coefficients, whose varying diagonal is what a Jacobi
+    preconditioner of the inner solve acts on.  coef: "const" (kappa = 1), "jump" (2x2x2 cell blocks, kappa 1 or 1e3
+    at random) or "lognormal" (kappa = exp(N(0, sigma^2)) per cell).  mass: B = a random positive diagonal,
+    uniform in [0.5, 2]; else B = None.  Lexicographic order i + m (j + m k), like the lattice generators."""
+    import scipy.sparse as sp
+
+    n = m ** 3
+    rng = np.random.default_rng(seed)
+    if coef == "const":
+        kap = np.ones(n)
+    elif coef == "jump":
+        h = m // 2 + 1
+        blk = rng.integers(0, 2, size=(h, h, h)).repeat(2, 0).repeat(2, 1).repeat(2, 2)[:m, :m, :m]
+        kap = np.where(blk.ravel() == 1, 1e3, 1.0)
+    elif coef == "lognormal":
+        kap = np.exp(rng.normal(0.0, sigma, n))
+    else:
+        raise ValueError(f"diffusion7_var: coef {coef!r}")
+    K = kap.reshape(m, m, m)                      # K[k, j, i]: cell i + m (j + m k)
+    idx = np.arange(n).reshape(m, m, m)
+    diag = np.zeros(n)
+    rows, cols, vals = [], [], []
+    for ax in range(3):
+        lo = [slice(None)] * 3; hi = [slice(None)] * 3
+        lo[ax] = slice(0, m - 1); hi[ax] = slice(1, m)
+        ka, kb = K[tuple(lo)], K[tuple(hi)]
+        t = (2.0 * ka * kb / (ka + kb)).ravel()
+        ia, ib = idx[tuple(lo)].ravel(), idx[tuple(hi)].ravel()
+        rows += [ia, ib]; cols += [ib, ia]; vals += [-t, -t]
+        np.add.at(diag, ia, t); np.add.at(diag, ib, t)
+        f0 = [slice(None)] * 3; f1 = [slice(None)] * 3
+        f0[ax] = 0; f1[ax] = m - 1
+        diag[idx[tuple(f0)].ravel()] += 2.0 * K[tuple(f0)].ravel()
+        diag[idx[tuple(f1)].ravel()] += 2.0 * K[tuple(f1)].ravel()
+    rows.append(np.arange(n)); cols.append(np.arange(n)); vals.append(diag)
+    A = sp.csc_matrix((np.concatenate(vals), (np.concatenate(rows), np.concatenate(cols))), shape=(n, n))
+    A.sum_duplicates(); A.sort_indices()
+
+    def ccs(M):
+        return CCS(n, n, M.indptr.astype(np.int32), M.indices.astype(np.int32), M.data.astype(np.float64))
+
+    B = None
+    if mass:
+        B = ccs(sp.diags(np.random.default_rng(seed + 1).uniform(0.5, 2.0, n)).tocsc())
+    return Pencil("diffusion7_var", ccs(A), B, {"m": m, "n": n, "coef": coef, "seed": seed, "sigma": sigma, "mass": mass})
+
+
 def _tensor27(m: int, ax, ay, az, scale_terms):
     """sum over terms of (X (x) Y (x) Z) with 1-D tridiagonal factors given as (lo, di, up)."""
     offs, coefs = [], []

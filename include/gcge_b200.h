@@ -240,6 +240,13 @@ typedef struct b200_bpcg_params_ {
 int b200_block_pcg(const b200_mat *A, const b200_mat *B, b200_mv *b, b200_mv *x,
                    const int *start, const int *end, const b200_bpcg_params *prm,
                    b200_mv *ws_r, b200_mv *ws_p, b200_mv *ws_w, int *niter, double *residual);
+/* The same with a preconditioner: pc = 0 none (== b200_block_pcg), 1 point Jacobi with D = diag(A + shift B)
+ * (B NULL: diag(A) + shift).  rho = r^T D^-1 r drives alpha and beta, p = D^-1 r + beta p; the residual norms, the
+ * stop test and *residual stay on ||r||_2, so rate / tol mean what they mean without it.  Fails, with x untouched,
+ * when a row of A (or B) stores no diagonal entry or the diagonal of A + shift B is not > 0. */
+int b200_block_pcg_pc(const b200_mat *A, const b200_mat *B, b200_mv *b, b200_mv *x,
+                      const int *start, const int *end, const b200_bpcg_params *prm, int pc,
+                      b200_mv *ws_r, b200_mv *ws_p, b200_mv *ws_w, int *niter, double *residual);
 
 /* All eigenpairs of the symmetric n x n host matrix a (column-major, lda; upper or lower
  * triangle both read), ascending; on-device parallel-order Jacobi.  Replaces the dsyevx
@@ -265,6 +272,9 @@ typedef struct b200_gcg_params_ {
 	/* 0 "mgs" (b200_mv_orth), 1 "bgs" (b200_mv_orth_bgs): -gcge_{initX,compP,compW}_orth_method,
 	 * reference src/ops_eig_sol_gcg.c:1757-1785 */
 	int    initX_orth_method, compP_orth_method, compW_orth_method;
+	/* preconditioner of the inner BlockPCG (b200_block_pcg_pc): 0 none (the reference's), 1 Jacobi with the sigma
+	 * of each ComputeW / ComputeW12 call */
+	int    compW_cg_pc;
 } b200_gcg_params;
 typedef struct b200_gcg_stats_ {
 	int    numIter, nevConv;
