@@ -22,14 +22,13 @@
 // false instantiations are the unpreconditioned kernels unchanged.
 #include "b200_stream.cuh"
 
-constexpr int BPCG_CTAS_MAX = 8;                 // buffers are sized for this many CTAs per SM
-// CTAs per SM the streaming kernels of the CG step are cut into (option bpcg_ctas, 1 ... 8; measured: profiles/)
-static inline int bpcg_ctas() { const int v = b200_opt(B200_OPT_BPCG_CTAS); return (v >= 1 && v <= BPCG_CTAS_MAX) ? v : 6; }
-#define BPCG_CTAS_PER_SM bpcg_ctas()
+// CTAs per SM the streaming kernels of the CG step are cut into; the partial buffers are sized for it (measured
+// flat between 3 and 8: profiles/)
+constexpr int BPCG_CTAS_PER_SM = 6;
 
 extern "C" int b200k_bpcg_state(int k, b200_bpcg_state *st)
 {
-	const int chunks_max = g_b200.num_sms * BPCG_CTAS_MAX + 8;
+	const int chunks_max = g_b200.num_sms * BPCG_CTAS_PER_SM + 8;
 	const size_t dbl = (size_t)10 * k + (size_t)chunks_max * 3 * k;
 	const size_t bytes = sizeof(double) * dbl + sizeof(int) * ((size_t)k + 8) + 64;
 	char *base = (char *)b200_scratch(4, bytes);

@@ -349,7 +349,7 @@ gram_tma2_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant_
 static int gram_tma2_launch(long long n, int p, int q, const double *x, int ldx, const double *y, int ldy,
                             long long rows_per_chunk, dim3 grid, int lower, double *part)
 {
-	if (b200_opt(B200_OPT_NO_TMA_DENSE) || n < G2_BK || n > 0x7fffffffLL || ((uintptr_t)x % 16) || ((uintptr_t)y % 16) || (ldx & 1) || (ldy & 1)) return 2;
+	if (n < G2_BK || n > 0x7fffffffLL || ((uintptr_t)x % 16) || ((uintptr_t)y % 16) || (ldx & 1) || (ldy & 1)) return 2;
 	tmap_encode_fn enc = tmap_encoder();
 	if (!enc) return 2;
 	CUtensorMap tmx, tmy;
@@ -841,7 +841,7 @@ lincomb_tma_kernel(const __grid_constant__ CUtensorMap tmx, long long n, int p, 
 static int lincomb_tma_launch(long long n, int p, int q, const double *x, int ldx, const double *c_dev, int c_rs, int c_cs,
                               const double *beta_dev, int incb, double *y, int ldy)
 {
-	if (b200_opt(B200_OPT_NO_TMA_DENSE) || n < LC_BM || c_cs != 1 || (c_rs & 1) || (q & 1) || ((uintptr_t)c_dev % 16) || ((uintptr_t)x % 16) || (ldx & 1) ||
+	if (n < LC_BM || c_cs != 1 || (c_rs & 1) || (q & 1) || ((uintptr_t)c_dev % 16) || ((uintptr_t)x % 16) || (ldx & 1) ||
 	    n > 0x7fffffffLL)
 		return 2;
 	tmap_encode_fn enc = tmap_encoder();

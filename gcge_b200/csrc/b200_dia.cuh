@@ -1,9 +1,22 @@
 // Device pieces shared by the diagonal-image SpMM kernels (b200_spmm.cu: 1-D row blocks; b200_spmm_lat.cu:
 // lattice tiles marching through the planes).
 #pragma once
+#include "b200_internal.h"
 #include "b200_tma.cuh"
 
 constexpr int DIA_WMAX = 3;                            // widest run of consecutive offsets
+
+// The block widths k = 2 KP with a compile-time kernel, X(KP) for each: they select the warp-specialised 1-D kernel
+// (b200_spmm.cu), the lattice kernel and the multi-rank overlap path; other widths take the generic kernels.
+#define DIA_WS_WIDTHS(X) X(4) X(5) X(6) X(8) X(10) X(12) X(15) X(16) X(20) X(24) X(25) X(28) X(30) X(32)
+
+// the run of M's diagonal image that holds offset 0 (the main diagonal); -1: none
+static inline int dia_zero_run(const b200_mat *M)
+{
+	for (int g = 0; g < M->dia_ng; ++g)
+		if (M->dia_off_h[g] <= 0 && M->dia_off_h[g] + M->dia_grp_h[2 * g + 1] > 0) return g;
+	return -1;
+}
 
 // One run of width W on the RB rows of a row group: x rows t = 0 .. RB + W - 2 of the run's box are read once
 // (128-bit) and x row t feeds matrix rows t - j, j < W.  The run's values of a matrix row sit 16-byte aligned

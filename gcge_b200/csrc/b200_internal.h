@@ -68,15 +68,11 @@ int b200k_lat_detect(b200_mat *A);
 int b200k_spmm_lat(const b200_mat *M, const double *x, int ldx, double *y, int ldy, int k, const int *gate,
                    double *dot_part, int dot_cap, int *nparts, int mode);
 
-// ---- run-time switches (b200_runtime.cu): one table, filled ONCE from the environment (B200_<NAME>) at b200_init,
-// changeable through b200_option_set / the OPS adaptor's -b200_<name> command-line options; kernels read the cached ints
-enum { B200_OPT_NO_DIA = 0, B200_OPT_NO_LAT, B200_OPT_SPMM_OLD_DIA, B200_OPT_NO_FUSED_DOT, B200_OPT_NO_TMA_DENSE,
-       B200_OPT_HOST_BUILD, B200_OPT_NO_OVERLAP, B200_OPT_NO_P2P, B200_OPT_NO_KERNEL_ALLREDUCE, B200_OPT_SYEV_PROF,
-       B200_OPT_BPCG_TRACE, B200_OPT_SPMM_CTAS, B200_OPT_SPMM_NS, B200_OPT_LAT_TI, B200_OPT_LAT_TJ, B200_OPT_LAT_NS,
-       B200_OPT_LAT_EVEN_PITCH, B200_OPT_LAT_NO_VPAD, B200_OPT_LAT_VERBOSE, B200_OPT_LAT_NO_CONST, B200_OPT_ORTH_TRACE, B200_OPT_NO_AXPBY_BATCH, B200_OPT_BPCG_CTAS, B200_OPT_COUNT };
+// ---- run-time switches (b200_runtime.cu; the list is B200_OPTIONS in b200_dev.h): one table, filled ONCE from the
+// environment (B200_<NAME>) at b200_init, changeable through b200_option_set / the OPS adaptor's -b200_<name>
+// command-line options; kernels read the cached ints
 extern int g_b200_opt[B200_OPT_COUNT];
 static inline int b200_opt(int id) { return g_b200_opt[id]; }
-static_assert(B200_OPT_BPCG_TRACE == B200K_OPT_BPCG_TRACE && B200_OPT_ORTH_TRACE == B200K_OPT_ORTH_TRACE, "b200_dev.h option id out of step");
 
 extern b200_ctx g_b200;
 static inline bool b200_multi() { return g_b200.nranks > 1; }

@@ -55,9 +55,10 @@ extern "C" int b200_init(int device)
 // ---- run-time switches -------------------------------------------------------------------------------------
 int g_b200_opt[B200_OPT_COUNT];
 static const char *const g_opt_names[B200_OPT_COUNT] = {
-	"no_dia", "no_lat", "spmm_old_dia", "no_fused_dot", "no_tma_dense", "host_build", "no_overlap", "no_p2p",
-	"no_kernel_allreduce", "syev_prof", "bpcg_trace", "spmm_ctas", "spmm_ns", "lat_ti", "lat_tj", "lat_ns",
-	"lat_even_pitch", "lat_no_vpad", "lat_verbose", "lat_no_const", "orth_trace", "no_axpby_batch", "bpcg_ctas"};
+#define OPT_NAME(id, name) #name,
+	B200_OPTIONS(OPT_NAME)
+#undef OPT_NAME
+};
 
 // B200_<NAME> in the environment: a number is taken as is, anything else (incl. an empty value) means 1
 static void options_from_environment(void)

@@ -264,6 +264,12 @@ spmm_csr_block_kernel(int nrows, const int *__restrict__ rp, const int *__restri
 	}
 }
 
+// 16-byte accesses to x and y: both 16-byte aligned, even leading dimensions, an even number of columns
+static inline bool spmm_aligned16(const double *x, int ldx, const double *y, int ldy, int k)
+{
+	return (((uintptr_t)x | (uintptr_t)y) % 16 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (k % 2 == 0);
+}
+
 template <int G, int U>
 static int launch_spmm_block(int nrows, const int *rp, const int *ci, const double *va,
                              const double *x, int ldx, double *y, int ldy, int k, const int *gate, int rw)
@@ -271,8 +277,7 @@ static int launch_spmm_block(int nrows, const int *rp, const int *ci, const doub
 	const int R = 8 * (32 / G) * rw;
 	const unsigned grid = (unsigned)(((long long)nrows + R - 1) / R);
 	const size_t smem = sizeof(double2) * SPMM_CAP + sizeof(int) * ((size_t)R + 1);
-	const bool vec = (((uintptr_t)x | (uintptr_t)y) % 16 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (k % 2 == 0);
-	if (vec) spmm_csr_block_kernel<G, true, U><<<grid, 256, smem, g_b200.stream>>>(nrows, rp, ci, va, x, ldx, y, ldy, k, gate, rw);
+	if (spmm_aligned16(x, ldx, y, ldy, k)) spmm_csr_block_kernel<G, true, U><<<grid, 256, smem, g_b200.stream>>>(nrows, rp, ci, va, x, ldx, y, ldy, k, gate, rw);
 	else     spmm_csr_block_kernel<G, false, U><<<grid, 256, smem, g_b200.stream>>>(nrows, rp, ci, va, x, ldx, y, ldy, k, gate, rw);
 	B200_KERNEL_CHECK();
 	return 0;
@@ -295,8 +300,7 @@ static int launch_spmm_wide(int nrows, const int *rp, const int *ci, const doubl
 {
 	const int rows_per_cta = 8 * (32 / G);
 	const unsigned grid = (unsigned)(((long long)nrows + rows_per_cta - 1) / rows_per_cta);
-	const bool vec = (((uintptr_t)x | (uintptr_t)y) % 16 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (k % 2 == 0);
-	if (vec) spmm_csr_wide_kernel<G, NPASS, true, 4><<<grid, 256, 0, g_b200.stream>>>(nrows, rp, ci, va, x, ldx, y, ldy, k, gate);
+	if (spmm_aligned16(x, ldx, y, ldy, k)) spmm_csr_wide_kernel<G, NPASS, true, 4><<<grid, 256, 0, g_b200.stream>>>(nrows, rp, ci, va, x, ldx, y, ldy, k, gate);
 	else     spmm_csr_wide_kernel<G, NPASS, false, 4><<<grid, 256, 0, g_b200.stream>>>(nrows, rp, ci, va, x, ldx, y, ldy, k, gate);
 	B200_KERNEL_CHECK();
 	return 0;
@@ -453,6 +457,22 @@ spmm_dia_tma_kernel(const __grid_constant__ CUtensorMap tmx, int nrows, int nblo
 	}
 }
 
+// 2-D tensor map of the x window of the 1-D diagonal kernels: dim0 = the k columns, dim1 = the hb + nloc + ha rows
+// (halo rows in front of and behind the local rows), box = (k, box_rows).  false: not available
+static bool dia_x_tmap(CUtensorMap *tm, const b200_mat *M, const double *x, int ldx, int k, int box_rows)
+{
+	tmap_encode_fn enc = tmap_encoder();
+	if (!enc) return false;
+	const double *base = x - (size_t)M->halo_below * ldx;   // first row of the window
+	const cuuint64_t gdim[2] = {(cuuint64_t)k, (cuuint64_t)(M->nrows + M->nhalo)};
+	const cuuint64_t gstr[1] = {(cuuint64_t)ldx * 8};
+	const cuuint32_t box[2] = {(cuuint32_t)k, (cuuint32_t)box_rows};
+	const cuuint32_t estr[2] = {1, 1};
+	return enc(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double *>(base), gdim, gstr, box, estr,
+	           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+	           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 // returns 0 launched, 1 error, 2 not applicable (caller falls back to the CSR kernels)
 template <int G, int RB, int NS>
 static int launch_spmm_dia(const b200_mat *M, const double *x, int ldx, double *y, int ldy, int k, const int *gate)
@@ -463,19 +483,9 @@ static int launch_spmm_dia(const b200_mat *M, const double *x, int ldx, double *
 	const int tile_bytes = (((ROWS + DIA_WMAX - 1) * k * 8) + 127) & ~127;
 	const size_t smem = (size_t)NS * tile_bytes + 2 * (size_t)ROWS * nd * 8;
 	if (smem > 200 * 1024) return 2;
-	tmap_encode_fn enc = tmap_encoder();
-	if (!enc) return 2;
-	const int hb = M->halo_below, span = M->nrows + M->nhalo;
-	const double *base = x - (size_t)hb * ldx;               // first row of the window
 	CUtensorMap tm;
-	const cuuint64_t gdim[2] = {(cuuint64_t)k, (cuuint64_t)span};
-	const cuuint64_t gstr[1] = {(cuuint64_t)ldx * 8};
-	const cuuint32_t box[2] = {(cuuint32_t)k, (cuuint32_t)(ROWS + DIA_WMAX - 1)};
-	const cuuint32_t estr[2] = {1, 1};
-	const CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double *>(base), gdim, gstr, box, estr,
-	                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-	                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-	if (r != CUDA_SUCCESS) return 2;
+	if (!dia_x_tmap(&tm, M, x, ldx, k, ROWS + DIA_WMAX - 1)) return 2;
+	const int hb = M->halo_below;
 	static bool attr_set = false;
 	if (!attr_set) {
 		B200_CUDA(cudaFuncSetAttribute(spmm_dia_tma_kernel<G, RB, NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
@@ -673,29 +683,18 @@ static int launch_spmm_dia_ws(const b200_mat *M, const double *x, int ldx, doubl
 	const int ng = M->dia_ng, nd = M->dia_ndp;
 	const int tile_bytes = (((ROWS + DIA_WMAX - 1) * K * 8) + 127) & ~127;
 	const size_t val_smem = 2 * (size_t)ROWS * nd * 8;
-	// ring depth: the deepest that still lets `want_ctas` CTAs share an SM (measured at k = 40: three
+	// ring depth: the deepest that still lets MINB CTAs share an SM (measured at k = 40: three
 	// CTAs with 3 tiles each 0.201 ms, two with 6 tiles 0.205 ms, one with 8 tiles 0.29 ms, four with
 	// 2 tiles 0.32 ms)
-	const int want_ctas = b200_opt(B200_OPT_SPMM_CTAS) > 0 ? b200_opt(B200_OPT_SPMM_CTAS) : MINB, ns_env = b200_opt(B200_OPT_SPMM_NS);
-	const size_t budget = (size_t)(224 * 1024) / (want_ctas > 0 ? want_ctas : 1) - 2048;
-	int NS = ns_env > 0 ? ns_env : (budget > val_smem ? (int)((budget - val_smem) / tile_bytes) : 0);
+	const size_t budget = (size_t)(224 * 1024) / MINB - 2048;
+	int NS = budget > val_smem ? (int)((budget - val_smem) / tile_bytes) : 0;
 	if (NS > DIA2_MAX_NS) NS = DIA2_MAX_NS;
 	if (NS < 2) NS = 2;
 	const size_t smem = (size_t)NS * tile_bytes + val_smem;
 	if (smem > 200 * 1024) return 2;
-	tmap_encode_fn enc = tmap_encoder();
-	if (!enc) return 2;
-	const int hb = M->halo_below, span = M->nrows + M->nhalo;
-	const double *base = x - (size_t)hb * ldx;               // first row of the window
 	CUtensorMap tm;
-	const cuuint64_t gdim[2] = {(cuuint64_t)K, (cuuint64_t)span};
-	const cuuint64_t gstr[1] = {(cuuint64_t)ldx * 8};
-	const cuuint32_t box[2] = {(cuuint32_t)K, (cuuint32_t)(ROWS + DIA_WMAX - 1)};
-	const cuuint32_t estr[2] = {1, 1};
-	const CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double *>(base), gdim, gstr, box, estr,
-	                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-	                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-	if (r != CUDA_SUCCESS) return 2;
+	if (!dia_x_tmap(&tm, M, x, ldx, K, ROWS + DIA_WMAX - 1)) return 2;
+	const int hb = M->halo_below;
 	static bool attr_set = false;
 	if (!attr_set) {
 		B200_CUDA(cudaFuncSetAttribute(spmm_dia_ws_kernel<KP, CP, RB, NT, DOT, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
@@ -760,44 +759,31 @@ static int launch_spmm_dia_ws_kp(const b200_mat *M, const double *x, int ldx, do
 static bool dia_ws_has(int k)
 {
 	switch (k) {
-	case 8: case 10: case 12: case 16: case 20: case 24: case 30: case 32: case 40: case 48: case 50: case 56: case 60: case 64:
-		return !b200_opt(B200_OPT_SPMM_OLD_DIA);
+#define HAS(KP_) case 2 * KP_:
+	DIA_WS_WIDTHS(HAS) return true;
+#undef HAS
 	default: return false;
 	}
 }
 
-// The block widths with a compile-time kernel; anything else takes the generic kernel above.
+// The block widths with a compile-time kernel (DIA_WS_WIDTHS); anything else takes the generic kernel above.
 // One column pair per lane, 8 consumer warps, three CTAs per SM: measured best at every width
 // (n = 1 M P1-FEM, k = 40: 0.204 ms; two pairs per lane 0.226 ms; 4-warp CTAs 0.216 - 0.249 ms;
 // gpurun_out/spmm_variants3.log, summarised in profiles/).
 static int spmm_dia_ws_dispatch(const b200_mat *M, const double *x, int ldx, double *y, int ldy, int k, const int *gate,
                                 double *dot_part, int dot_cap, int *nparts, int mode = 0)
 {
-	if (b200_opt(B200_OPT_SPMM_OLD_DIA)) return 2;
 	{
 		// lattice operators: plane tiles marching along k (b200_spmm_lat.cu); same bits, fewer shared-memory bytes
 		const int rc = b200k_spmm_lat(M, x, ldx, y, ldy, k, gate, dot_part, dot_cap, nparts, mode);
 		if (rc != 2) return rc;
 	}
-#define WS(KP_) launch_spmm_dia_ws_kp<KP_, 1>(M, x, ldx, y, ldy, gate, dot_part, dot_cap, nparts, mode)
 	switch (k) {
-	case 8:  return WS(4);
-	case 10: return WS(5);
-	case 12: return WS(6);
-	case 16: return WS(8);
-	case 20: return WS(10);
-	case 24: return WS(12);
-	case 30: return WS(15);
-	case 32: return WS(16);
-	case 40: return WS(20);
-	case 48: return WS(24);
-	case 50: return WS(25);
-	case 56: return WS(28);
-	case 60: return WS(30);
-	case 64: return WS(32);
+#define WS(KP_) case 2 * KP_: return launch_spmm_dia_ws_kp<KP_, 1>(M, x, ldx, y, ldy, gate, dot_part, dot_cap, nparts, mode);
+	DIA_WS_WIDTHS(WS)
+#undef WS
 	default: return 2;
 	}
-#undef WS
 }
 
 // ---- diagonal image, 1 ... 4 columns ---------------------------------------------------------------------------
@@ -861,8 +847,7 @@ static int launch_spmm_dia_narrow(const b200_mat *M, const double *x, int ldx, d
 // diagonal image, at most 64 columns
 static int spmm_dia_dispatch(const b200_mat *M, const double *x, int ldx, double *y, int ldy, int k, const int *gate)
 {
-	const bool vec = (((uintptr_t)x | (uintptr_t)y) % 16 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (k % 2 == 0);
-	if (!vec) return 2;
+	if (!spmm_aligned16(x, ldx, y, ldy, k)) return 2;
 	{
 		const int rc = spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, nullptr, 0, nullptr);
 		if (rc != 2) return rc;
@@ -965,36 +950,38 @@ static int spmm_csr_local(const b200_mat *M, int trans, const double *x, int ldx
 static bool spmm_overlap_ok(const b200_mat *M, int trans, const double *x, int ldx, const double *y, int ldy, int k)
 {
 	if (!b200_multi() || trans || M->nnbr == 0 || M->dia_nd <= 0 || M->nrows <= 0 || !g_b200.comm_stream) return false;
-	const bool vec = (((uintptr_t)x | (uintptr_t)y) % 16 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (k % 2 == 0);
-	if (!vec || !dia_ws_has(k)) return false;
+	if (!spmm_aligned16(x, ldx, y, ldy, k) || !dia_ws_has(k)) return false;
 	// the dot partials of the two launches must fit the caller's buffer: at most 4 CTAs per SM each
 	return b200k_p2p_usable(M, k) != 0;
 }
 
-int b200k_spmm(const b200_mat *M, int trans, const double *x, int ldx, double *y, int ldy, int k,
-               const int *gate)
+// y = A x (b200k_spmm) or, with dot_part, y = A x and the per-CTA partials of diag(x^T w) through the warp-specialised
+// diagonal kernel (b200k_spmm_dot, which has checked that it applies): the halo exchange (several ranks: copy engines
+// overlapped with the interior blocks, or NCCL), the profiler scope and the launches.  Returns that kernel's 2 when it
+// does not take the block after all.
+static int spmm_body(const b200_mat *M, int trans, const double *x, int ldx, double *y, int ldy, int k, const int *gate,
+                     double *dot_part, int dot_cap, int *nparts)
 {
-	if (trans && !M->t_rp) {
-		// row-partitioned matrix: only the forward image is kept; A^T x == A x when A is symmetric
-		// (the reference assumes that for every matrix, app/app_ccs.c:140-150)
-		B200_CHECK(M->symmetric, "transposed SpMM of a non-symmetric matrix is not available across ranks");
-		trans = 0;
-	}
 	const int nrows = trans ? M->ncols : M->nrows;
-	if (k <= 0) return 0;
+	const double bytes = 12.0 * M->nnz + 4.0 * (nrows + 1) + 8.0 * k * ((double)M->nrows + M->ncols);
+	const double flops = dot_part ? 2.0 * M->nnz * k + 2.0 * M->nrows * k : 2.0 * M->nnz * k;
 	if (spmm_overlap_ok(M, trans, x, ldx, y, ldy, k)) {
 		// the halo rows travel on the comm stream (copy engines) while the interior blocks multiply
 		if (b200k_p2p_halo_exchange(M, const_cast<double *>(x), ldx, k)) return 1;
-		B200Prof prof(B200_PROF_SPMM, 12.0 * M->nnz + 4.0 * (nrows + 1) + 8.0 * k * ((double)M->nrows + M->ncols),
-		              2.0 * M->nnz * k);
-		if (spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, nullptr, 0, nullptr, 1)) return 1;
+		B200Prof prof(B200_PROF_SPMM, bytes, flops);
+		int n1 = 0, n2 = 0;
+		if (spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, dot_part, dot_cap, &n1, 1)) return 1;
 		B200_CUDA(cudaStreamWaitEvent(g_b200.stream, g_b200.ev_halo_done, 0));
-		return spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, nullptr, 0, nullptr, 2) ? 1 : 0;
+		if (spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, dot_part ? dot_part + (size_t)n1 * k : nullptr, dot_cap - n1,
+		                         &n2, 2))
+			return 1;
+		if (dot_part) *nparts = n1 + n2;
+		return 0;
 	}
 	if (b200_multi() && halo_exchange(M, const_cast<double *>(x), ldx, k)) return 1;
 	if (nrows <= 0) return 0;
-	B200Prof prof(B200_PROF_SPMM, 12.0 * M->nnz + 4.0 * (nrows + 1) + 8.0 * k * ((double)M->nrows + M->ncols),
-	              2.0 * M->nnz * k);
+	B200Prof prof(B200_PROF_SPMM, bytes, flops);
+	if (dot_part) return spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, dot_part, dot_cap, nparts);
 	if (!trans && M->dia_nd > 0 && M->nrows > 0) {
 		// diagonal image, 64 columns per pass (1 ... 4 columns: the narrow kernel); whatever it cannot take
 		// (a misaligned or odd block) goes to the CSR kernels
@@ -1012,6 +999,19 @@ int b200k_spmm(const b200_mat *M, int trans, const double *x, int ldx, double *y
 	return spmm_csr_local(M, trans, x, ldx, y, ldy, k, gate);
 }
 
+int b200k_spmm(const b200_mat *M, int trans, const double *x, int ldx, double *y, int ldy, int k,
+               const int *gate)
+{
+	if (trans && !M->t_rp) {
+		// row-partitioned matrix: only the forward image is kept; A^T x == A x when A is symmetric
+		// (the reference assumes that for every matrix, app/app_ccs.c:140-150)
+		B200_CHECK(M->symmetric, "transposed SpMM of a non-symmetric matrix is not available across ranks");
+		trans = 0;
+	}
+	if (k <= 0) return 0;
+	return spmm_body(M, trans, x, ldx, y, ldy, k, gate, nullptr, 0, nullptr);
+}
+
 // w = A x together with the per-CTA partial sums of diag(x^T w) (fused BlockPCG step).  Only the
 // warp-specialised diagonal kernel can do this; returns 2 (nothing launched) when it does not
 // apply, and the caller runs the plain SpMM followed by the streaming dot kernel.
@@ -1020,30 +1020,10 @@ int b200k_spmm_dot(const b200_mat *M, const double *x, int ldx, double *y, int l
 {
 	*nparts = 0;
 	if (!(M->dia_nd > 0 && k > 4 && k <= 64 && M->nrows > 0) || b200_opt(B200_OPT_NO_FUSED_DOT)) return 2;
-	{
-		// the epilogue takes p from the run that holds offset 0 (the main diagonal): without one, no fusion
-		bool has_diag = false;
-		for (int g = 0; g < M->dia_ng; ++g)
-			has_diag = has_diag || (M->dia_off_h[g] <= 0 && M->dia_off_h[g] + M->dia_grp_h[2 * g + 1] > 0);
-		if (!has_diag) return 2;
-	}
-	const bool vec = (((uintptr_t)x | (uintptr_t)y) % 16 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (k % 2 == 0);
-	if (!vec) return 2;
-	if (spmm_overlap_ok(M, 0, x, ldx, y, ldy, k)) {
-		if (b200k_p2p_halo_exchange(M, const_cast<double *>(x), ldx, k)) return 1;
-		B200Prof prof(B200_PROF_SPMM, 12.0 * M->nnz + 4.0 * (M->nrows + 1) + 8.0 * k * ((double)M->nrows + M->ncols),
-		              2.0 * M->nnz * k + 2.0 * M->nrows * k);
-		int n1 = 0, n2 = 0;
-		if (spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, dot_part, dot_cap, &n1, 1)) return 1;
-		B200_CUDA(cudaStreamWaitEvent(g_b200.stream, g_b200.ev_halo_done, 0));
-		if (spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, dot_part + (size_t)n1 * k, dot_cap - n1, &n2, 2)) return 1;
-		*nparts = n1 + n2;
-		return 0;
-	}
-	if (b200_multi() && halo_exchange(M, const_cast<double *>(x), ldx, k)) return 1;
-	B200Prof prof(B200_PROF_SPMM, 12.0 * M->nnz + 4.0 * (M->nrows + 1) + 8.0 * k * ((double)M->nrows + M->ncols),
-	              2.0 * M->nnz * k + 2.0 * M->nrows * k);
-	return spmm_dia_ws_dispatch(M, x, ldx, y, ldy, k, gate, dot_part, dot_cap, nparts);
+	// the epilogue takes p from the run that holds offset 0 (the main diagonal): without one, no fusion
+	if (dia_zero_run(M) < 0) return 2;
+	if (!spmm_aligned16(x, ldx, y, ldy, k)) return 2;
+	return spmm_body(M, 0, x, ldx, y, ldy, k, gate, dot_part, dot_cap, nparts);
 }
 
 extern "C" int b200_mat_dot_multivec(const b200_mat *A, int trans, const b200_mv *x, b200_mv *y,

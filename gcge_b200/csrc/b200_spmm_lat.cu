@@ -300,9 +300,7 @@ int b200k_lat_detect(b200_mat *A)
 	if (A->dia_nd <= 0 || A->nrows <= 0 || b200_opt(B200_OPT_NO_LAT)) return 0;
 	const long long n = A->nrows_global;
 	// the central run must hold offset 0; s1 comes from the first run above it, s2 from the runs beyond
-	int zc = -1;
-	for (int g = 0; g < A->dia_ng; ++g)
-		if (A->dia_off_h[g] <= 0 && A->dia_off_h[g] + A->dia_grp_h[2 * g + 1] > 0) zc = g;
+	const int zc = dia_zero_run(A);
 	if (zc < 0 || zc + 1 >= A->dia_ng) return 0;
 	const long long a = A->dia_off_h[zc + 1];
 	long long best1 = 0, best2 = 0;
@@ -364,9 +362,8 @@ int b200k_lat_detect(b200_mat *A)
 // even pitch 22 every group boundary inside a quarter-warp is a two-way conflict, +24 % wavefronts on the x reads).
 static int lat_pitch(int TI, int K)
 {
-	const int force = b200_opt(B200_OPT_LAT_EVEN_PITCH);
 	int pitch = TI + 2;
-	if (!force && (K * 8) % 128 != 0 && pitch % 2 == 0) ++pitch;
+	if ((K * 8) % 128 != 0 && pitch % 2 == 0) ++pitch;
 	return pitch;
 }
 
@@ -377,8 +374,7 @@ static int lat_pitch(int TI, int K)
 // rows 4 apart 64 bytes apart; the tensor-map box is simply wider than the image and the padding arrives as zeros.
 static int lat_vpitch(int ndp)
 {
-	const int off = b200_opt(B200_OPT_LAT_NO_VPAD);
-	return (!off && ndp % 4 == 0) ? ndp + 2 : ndp;
+	return ndp % 4 == 0 ? ndp + 2 : ndp;
 }
 
 // returns 0 launched, 1 error, 2 not applicable; mode 0: all planes, 1: interior planes (no halo plane needed),
@@ -397,21 +393,17 @@ static int launch_spmm_lat(const b200_mat *M, const double *x, int ldx, double *
 	if (!lat_decompose(M, s1, s2, P.run, &P.zero_run, &P.zero_pos)) return 2;
 	if (DOT && P.zero_run < 0) return 2;
 	// ---- tile: TI x TJ rows of a plane, ring depth; estimated shared-memory cycles per matrix row decide
-	const int env_ti = b200_opt(B200_OPT_LAT_TI), env_tj = b200_opt(B200_OPT_LAT_TJ), env_ns = b200_opt(B200_OPT_LAT_NS);
 	const size_t smem_cap = 227 * 1024 - 1024;
 	int sum_reads = 0, n3 = 0;
 	for (int g = 0; g < P.ng; ++g) { sum_reads += LAT_RB + P.run[g].w - 1; n3 += P.run[g].w == 3; }
 	double best = 1e300; int bTI = 0, bTJ = 0, bNS = 0;
 	for (int TI = 8; TI <= 64; TI += LAT_RB) {
-		if (env_ti && TI != env_ti) continue;
 		for (int TJ = 1; TJ <= 16; ++TJ) {
-			if (env_tj && TJ != env_tj) continue;
 			// TMA destinations are 128-byte aligned
 			const int pitch = lat_pitch(TI, K);
 			const size_t slice = ((size_t)pitch * (TJ + 2) * K * 8 + 127) & ~(size_t)127;
 			const size_t vb = CONST ? 0 : (((size_t)TI * TJ * lat_vpitch(P.ndp) * 8 + 127) & ~(size_t)127);
 			for (int NS = 4; NS <= LAT_MAX_NS; ++NS) {
-				if (env_ns && NS != env_ns) continue;
 				const int NV = NS - 2;
 				if (NS * slice + NV * vb > smem_cap) continue;
 				const int nti = (s1 + TI - 1) / TI, ntj = (my + TJ - 1) / TJ;
@@ -445,9 +437,6 @@ static int launch_spmm_lat(const b200_mat *M, const double *x, int ldx, double *
 		P.run[g].rowoff = dj1 * P.pitch + di1;
 	}
 	const size_t smem = (size_t)P.NS * P.slice_stride + (size_t)P.NV * P.val_stride;
-	if (b200_opt(B200_OPT_LAT_VERBOSE))
-		fprintf(stderr, "spmm_lat k=%d dot=%d const=%d lattice %d x %d x %d: tile TI=%d TJ=%d pitch=%d ring %d + %d, %zu bytes smem, est %.1f wavefronts/row\n",
-		        K, (int)DOT, (int)CONST, s1, my, np, P.TI, P.TJ, P.pitch, P.NS, P.NV, smem, best);
 	// ---- tensor maps: x as (K, s1, my, planes) with a halo plane in front / behind where a slab neighbour exists
 	tmap_encode_fn enc = tmap_encoder();
 	if (!enc) return 2;
@@ -532,28 +521,14 @@ static int launch_spmm_lat_kp(const b200_mat *M, const double *x, int ldx, doubl
 	return launch_spmm_lat<KP, 480, false, false>(M, x, ldx, y, ldy, gate, nullptr, 0, nullptr, mode);
 }
 
-// the block widths with a compile-time kernel (those of the 1-D warp-specialised kernel)
 int b200k_spmm_lat(const b200_mat *M, const double *x, int ldx, double *y, int ldy, int k, const int *gate,
                    double *dot_part, int dot_cap, int *nparts, int mode)
 {
 	if (M->lat_s1 <= 0) return 2;
-#define LT(KP_) launch_spmm_lat_kp<KP_>(M, x, ldx, y, ldy, gate, dot_part, dot_cap, nparts, mode)
 	switch (k) {
-	case 8:  return LT(4);
-	case 10: return LT(5);
-	case 12: return LT(6);
-	case 16: return LT(8);
-	case 20: return LT(10);
-	case 24: return LT(12);
-	case 30: return LT(15);
-	case 32: return LT(16);
-	case 40: return LT(20);
-	case 48: return LT(24);
-	case 50: return LT(25);
-	case 56: return LT(28);
-	case 60: return LT(30);
-	case 64: return LT(32);
+#define LT(KP_) case 2 * KP_: return launch_spmm_lat_kp<KP_>(M, x, ldx, y, ldy, gate, dot_part, dot_cap, nparts, mode);
+	DIA_WS_WIDTHS(LT)
+#undef LT
 	default: return 2;
 	}
-#undef LT
 }

@@ -190,7 +190,9 @@ syev_block_jacobi_kernel(int n, int NB, double *Mg, double *Vg, double *jbuf, in
 	const int Np = NB * BJ_B, m = NB / 2;
 	const int vrb = (Np / BJ_T + 1) / 2;                   // V jobs take two 32-row tiles each
 	const int a_jobs = m * (m - 1) / 2, v_jobs = vrb * m;
-	// where the time goes (block 0's view, clock64 ticks): [0] phase 1, [1] barrier, [2] phase 2, [3] barrier
+	// where the time goes (block 0's view, clock64 ticks): [0] phase 1, [1] barrier, [2] phase 2, [3] barrier.
+	// Kept on every call: without these clock reads ptxas schedules the kernel differently and it runs 0.4 - 1.2 %
+	// slower at N = 400 - 480 (B200, 1000 W power limit), same bits.
 	long long cyc[6] = {0, 0, 0, 0, 0, 0}, t_prev = clock64();     // [4], [5]: tile load / rotations inside phase 1
 	auto lap = [&](int slot) { const long long t = clock64(); cyc[slot] += t - t_prev; t_prev = t; };
 	int sweep = 0, converged = 0;

@@ -45,7 +45,7 @@ static int bpcg_chunk(const b200_mat *A, const b200_mat *B, long long n,
 	if (b200k_bpcg_begin(n, &st, b, ldb, r, ldr, prm->tol, prm->tol_type == 1)) return 1;
 	/* B200_BPCG_TRACE=1 (diagnostic, synchronises every iteration): column-iterations really needed
 	 * vs. launched -- how much a compaction of the active columns could save */
-	const int trace = b200k_opt(B200K_OPT_BPCG_TRACE);
+	const int trace = b200k_opt(B200_OPT_BPCG_TRACE);
 	long long act_sum = 0, iters_run = 0;
 	int it = 0;
 	for (; it < prm->max_iter; ++it) {

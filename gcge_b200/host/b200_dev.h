@@ -92,10 +92,16 @@ void b200_gcg_free_cache(void);               /* b200_gcg.c: the solver's cached
 void *b200_scratch(int slot, size_t bytes);   /* growable device scratch; NULL on failure */
 void *b200_pinned(int slot, size_t bytes);    /* growable pinned host staging */
 int  b200k_num_sms(void);
-/* cached run-time switch (b200_runtime.cu; ids of b200_internal.h) for the host-side C drivers */
+/* Run-time switches (b200_runtime.cu, DESIGN.md §10), X(ID, name) each: the ids B200_OPT_<ID> and the names of
+ * b200_option_name both come from this one list.  b200k_opt: the cached value, for the host-side C drivers. */
+#define B200_OPTIONS(X)                                                                                            \
+	X(NO_DIA, no_dia) X(NO_LAT, no_lat) X(NO_FUSED_DOT, no_fused_dot) X(HOST_BUILD, host_build)                    \
+	X(NO_OVERLAP, no_overlap) X(NO_P2P, no_p2p) X(NO_KERNEL_ALLREDUCE, no_kernel_allreduce) X(SYEV_PROF, syev_prof) \
+	X(BPCG_TRACE, bpcg_trace) X(LAT_NO_CONST, lat_no_const) X(ORTH_TRACE, orth_trace) X(NO_AXPBY_BATCH, no_axpby_batch)
+#define B200_OPT_ID_(id, name) B200_OPT_##id,
+enum { B200_OPTIONS(B200_OPT_ID_) B200_OPT_COUNT };
+#undef B200_OPT_ID_
 int  b200k_opt(int id);
-#define B200K_OPT_BPCG_TRACE 10
-#define B200K_OPT_ORTH_TRACE 20
 
 /* synchronising small transfers */
 int b200k_d2h(void *host, const void *dev, size_t bytes);

@@ -127,7 +127,7 @@ int b200_mv_orth(b200_mv *x, int start_x, int *end_x, const b200_mat *B,
 			               sc_in, sc_out, x->dist))
 				return 1;
 			if (s1 > 0 && round >= 1 && round + 1 < max_rounds && b200k_d2h(&cmax, cmax_dev, sizeof(double))) return 1;
-			if (b200k_opt(B200K_OPT_ORTH_TRACE) && s1 > 0 && round >= 1)
+			if (b200k_opt(B200_OPT_ORTH_TRACE) && s1 > 0 && round >= 1)
 				fprintf(stderr, "orth: block at %d of %d columns, round %d: max |coef| on unit columns %.3e (another pass from %.3e)\n",
 				        s1, kb, round, cmax, again_tol);
 			e1 = s1 + n_live;
